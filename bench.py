@@ -15,6 +15,10 @@ One JSON line on stdout (rank 0).  `value` times the device-resident loop with C
 `e2e` times the same loop through the host-array VecEnv API (pinned host buffers, H2D + D2H every step);
 `roofline` is the world kernel (dominant launch) against the measured HBM copy bandwidth; `cpu_baseline` times
 the oracle (CPU restatement, the one thing bench.py may run from oracle/) on the host cores for a bounded sample.
+
+`--dump-outputs DIR` writes what the last timed step of the `value` loop handed its caller (observations, rewards,
+done flags, actions, values, log-probabilities; rank 0) as DIR/<name>.npy, so that two builds can be compared output
+for output on the same seeded inputs.
 """
 from __future__ import annotations
 
@@ -25,8 +29,11 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True          # the tree may be read-only; bench.py writes nothing into it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+
+DUMP_LIMIT_BYTES = 64 << 20
 
 METRIC = "Baoding env-steps/sec (1/2/4/8 B200, policy in loop) vs host MuJoCo SubprocVecEnv"
 UNIT = "env-steps/s"
@@ -210,6 +217,25 @@ def run_reference(args):
 
 
 # ------------------------------------------------------------------------------------------------------------
+def dump_outputs(path, stepper):
+    """What ``stepper.step()`` left for its caller after the last timed step - every sub-batch's results concatenated in world
+    order - as float32 DIR/<name>.npy. Above DUMP_LIMIT_BYTES in all, the same seeded sample of worlds is kept in every file."""
+    import numpy as np
+    import torch
+
+    outs = {"obs": stepper.obs, "reward": stepper.rewards, "done": stepper.dones, "actions": [o[0] for o in stepper.out],
+            "values": [o[1] for o in stepper.out], "log_prob": [o[2] for o in stepper.out]}
+    arrays = {k: torch.cat([t.float() for t in v]).cpu().numpy() for k, v in outs.items()}
+    n = stepper.num_envs
+    row_bytes = sum(a.nbytes for a in arrays.values()) // n
+    rows = slice(None)
+    if row_bytes * n > DUMP_LIMIT_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_LIMIT_BYTES // row_bytes, replace=False))
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), np.ascontiguousarray(a[rows]))
+
+
 def run_b200(args):
     import numpy as np
     import torch
@@ -333,6 +359,8 @@ def run_b200(args):
     pipe_ms = pe0.elapsed_time(pe1)
     pipe_launches = sum(hv.sim.launch_count for hv in halves) + pol.launch_count - lp0
     status |= halves[0].sim.status() | halves[1].sim.status()
+    if args.dump_outputs and rank == 0:                     # before the e2e leg below steps the same sub-batches again
+        dump_outputs(args.dump_outputs, stepper)
 
     # ---- e2e: the SB3-shaped host-array API, H2D + D2H inside the timed region -------------------------------
     # (1) one MyoVecEnv, synchronous loop: obs H2D -> policy -> actions D2H -> step_async (actions H2D) -> step_wait
@@ -570,7 +598,12 @@ def main():
     ap.add_argument("--ppo-steps", type=int, default=128, help="n_steps of the PPO iteration leg")
     ap.add_argument("--ppo-batch-worlds", type=int, default=2048, help="world sequences per minibatch")
     ap.add_argument("--ppo-epochs", type=int, default=10)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the B200 path; the reference arm has none")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     return run_reference(args) if args.impl == "reference" else run_b200(args)

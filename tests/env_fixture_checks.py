@@ -35,7 +35,13 @@ def fixtures():
 def _get(group, tag):
     f, meta = fixtures()
     pre = f"{group}/{tag}/"
-    return {k[len(pre):]: f[k] for k in f.files if k.startswith(pre)}, meta[group][tag]
+    d = {k[len(pre):]: f[k] for k in f.files if k.startswith(pre)}
+    if "obs_cols" in d:          # reset observations are stored in the columns the checks read; any other column reads as NaN
+        cols = d.pop("obs_cols")
+        obs = np.full((len(d["obs"]), int(cols.max()) + 1), np.nan)
+        obs[:, cols] = d["obs"]
+        d["obs"] = obs
+    return d, meta[group][tag]
 
 
 def _make(lib, device, meta, n, seed=0, **extra):

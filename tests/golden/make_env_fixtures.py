@@ -12,6 +12,7 @@ physics = the fp64 oracle) and driven through ``EnvironmentFactory.create(name, 
 
 All three host RNGs the reference draws from (env.np_random, numpy's global, ``random``) are seeded; the recorded streams
 are what make the fixtures reproducible. Only runs where /root/reference exists; the .npz travels with the repository.
+``shrink`` keeps the stored file under 1 MB (see its docstring).
 
     python tests/golden/make_env_fixtures.py
 """
@@ -24,15 +25,10 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-sys.path.insert(0, os.path.join(ROOT, "tests"))
-import shim  # noqa: E402
-
-shim.install()
-import envs  # noqa: E402,F401  (the reference's registrations)
-from envs.environment_factory import EnvironmentFactory  # noqa: E402
-from myosuite.envs.myo.myochallenge.baoding_v1 import Task  # noqa: E402
 
 M_RESET = 256
+STEP_KEEP = 0.4         # share of each tag's non-terminal step cases that is stored (shrink)
+BAODING_RESET_OBS = [23, 24, 29, 30, 35, 36, 38, 39]      # ball xy and target xy: the reset observation columns the checks read
 BAODING_TERMS = ("pos_dist_1", "pos_dist_2", "act_reg", "alive", "sparse", "solved", "done", "dense")
 POSE_TERMS = ("pose", "bonus", "penalty", "act_reg", "sparse", "solved", "done", "dense")
 REORIENT_TERMS = ("pos_dist", "rot_dist", "act_reg", "alive", "sparse", "solved", "done", "dense", "pos_dist_diff", "rot_dist_diff")
@@ -161,7 +157,45 @@ def step_cases(env_name, config, n_cases, seed, every=3, horizon=40):
     return stack(cases[:n_cases])
 
 
+def shrink(out, meta, seed=0):
+    """Cuts the recorded fixtures down to what tests/env_fixture_checks.py reads, so that the .npz stays under 1 MB:
+    step observations in float32 (the checks compare them to 2e-4); reset observations (float64: their distributions are
+    compared value by value) only in the columns the checks read (``obs_cols`` names them; pose resets keep none); of each
+    tag's step cases every terminal one and a seeded ``STEP_KEEP`` share of the others."""
+    rng = np.random.default_rng(seed)
+    out = dict(out)
+    for tag in meta["reset"]:
+        pre = f"reset/{tag}/"
+        obs = out.pop(pre + "obs")
+        if pre + "task" in out:
+            cols = np.array(BAODING_RESET_OBS)
+        elif pre + "goal_quat" in out:          # die: object and goal pose, their errors (obs[o0 : o0 + 18])
+            o0 = (out[pre + "qpos"].shape[1] - 7) + (out[pre + "qvel"].shape[1] - 6)
+            cols = np.arange(o0, o0 + 18)
+        else:
+            continue
+        out[pre + "obs"] = obs[:, cols]
+        out[pre + "obs_cols"] = cols.astype(np.int32)
+    for tag in meta["step"]:
+        pre = f"step/{tag}/"
+        done = np.asarray(out[pre + "done"], bool)
+        rest = np.flatnonzero(~done)
+        keep = np.sort(np.concatenate([np.flatnonzero(done), rng.choice(rest, int(np.ceil(STEP_KEEP * len(rest))), replace=False)]))
+        for k in [k for k in out if k.startswith(pre)]:
+            out[k] = out[k][keep]
+        out[pre + "obs"] = out[pre + "obs"].astype(np.float32)
+    return out
+
+
 def main():
+    global EnvironmentFactory
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    import shim
+
+    shim.install()                  # the reference's sources: imported here so that ``shrink`` imports without them
+    import envs  # noqa: F401  (the reference's registrations)
+    from envs.environment_factory import EnvironmentFactory
+    from myosuite.envs.myo.myochallenge.baoding_v1 import Task  # noqa: F401
     cur = json.load(open(os.path.join(ROOT, "myochallenge_b200", "assets", "curriculum", "baoding_winner.json")))["steps"]
     out = {}
     meta = {"reset": {}, "step": {}}
@@ -207,6 +241,7 @@ def main():
     for tag, name, cfg, n in step_sets:
         put("step", tag, name, cfg, step_cases(name, cfg, n, 900 + len(meta["step"])))
         print("step", tag, flush=True)
+    out = shrink(out, meta)
     out["meta"] = np.array(json.dumps(meta))
     path = os.path.join(HERE, "env_fixtures.npz")
     np.savez_compressed(path, **out)
