@@ -107,6 +107,7 @@ struct DevModel {
   int o_qpos, o_qvel, o_act, o_ctrl, o_warm, o_xpos, o_xmat, o_xipos, o_cdof, o_cinert, o_cdofdot,
       o_cfrc, o_M, o_tenL, o_tenV, o_tenJ, o_actF, o_bias, o_passive, o_qact, o_smooth, o_qaccs,
       o_qacc, o_qcon, o_actdot, o_grad, o_p, o_Mp, o_Ma, o_H, o_lim, o_con, o_row, o_misc, o_obs, o_wparam,
+      o_seg,   // the tendon phase's per-segment results (nseg x SEG_OUT words)
       scratch_words;
   const float* g_tables;     // global copy of the table block
   int tab_words;             // its size in words (multiple of 4); world scratch starts right after it

@@ -38,7 +38,7 @@ const myo::Model& myo_model_host(const myo_model* m);
 
 namespace myo {
 
-constexpr int kThreads = 448;   // up to 14 one-warp worlds per CTA (register cap 144)
+constexpr int kThreads = 512;   // up to 16 one-warp worlds per CTA (register cap 128: 16 warps fill the register file)
 
 // hand world w to the full-capacity kernel of this env step
 MYO_DI void redo_push(const BatchPtrs& b, int w, int kind) {
@@ -464,7 +464,7 @@ struct myo_batch {
   int64_t launches = 0;
   std::vector<void*> allocs;
   // world grouping: after every env step the worlds are sorted by the constraint rows of their last substep, and the next
-  // step walks them in that order, so the 14 worlds that share a CTA (and its phase barriers) carry similar loads
+  // step walks them in that order, so the worlds that share a CTA (and its phase barriers) carry similar loads
   bool sort_worlds = false;
   int *order[2] = {nullptr, nullptr}, *iota = nullptr, *keys_out = nullptr;
   void* sort_tmp = nullptr;
@@ -569,12 +569,16 @@ template <int G> int configure(myo_batch* b) {
   if (const char* ov = getenv("MYO_WPC")) { const int v = atoi(ov); if (v >= 1 && v < wpc) wpc = v; }   // development override
   while (wpc > 1 && wpc * world_bytes > max_smem) wpc--;
   if (wpc * world_bytes > max_smem) { set_error("one world's scratch exceeds shared memory per CTA"); return MYO_E_LIMIT; }
+  // a batch smaller than one CTA steps no padding worlds beside its own; the CTA keeps room for one full-capacity world (redo)
+  wpc = std::min(wpc, b->n);
+  const size_t full_bytes = (size_t)b->pm.dm_full.scratch_words * sizeof(float);
+  if (tab_bytes + full_bytes > prop.sharedMemPerBlockOptin) { set_error("model tables + one full-capacity world exceed shared memory per CTA"); return MYO_E_LIMIT; }
   b->wpc = wpc;
   b->tab_bytes = (int)tab_bytes;
   CK(cudaFuncSetAttribute(init_worlds_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tab_bytes));
   CK(cudaFuncSetAttribute(extract_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tab_bytes));
   b->threads = wpc * G;
-  b->smem = (int)(tab_bytes + wpc * world_bytes);
+  b->smem = (int)(tab_bytes + std::max(wpc * world_bytes, full_bytes));
   CK(cudaFuncSetAttribute(world_kernel<G>, cudaFuncAttributeMaxDynamicSharedMemorySize, b->smem));
   int per_sm = 0;
   CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, world_kernel<G>, b->threads, b->smem));
@@ -582,8 +586,6 @@ template <int G> int configure(myo_batch* b) {
   const int need = (b->n + wpc - 1) / wpc;
   b->grid = std::max(1, std::min(need, prop.multiProcessorCount * per_sm));
   // full-capacity kernel: one world per CTA
-  const size_t full_bytes = (size_t)b->pm.dm_full.scratch_words * sizeof(float);
-  if (tab_bytes + full_bytes > prop.sharedMemPerBlockOptin) { set_error("model tables + one full-capacity world exceed shared memory per CTA"); return MYO_E_LIMIT; }
   b->solo_smem = (int)(tab_bytes + full_bytes);
   CK(cudaFuncSetAttribute(solo_kernel<G>, cudaFuncAttributeMaxDynamicSharedMemorySize, b->solo_smem));
   cudaFuncAttributes fs;

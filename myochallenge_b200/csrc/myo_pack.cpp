@@ -578,7 +578,18 @@ std::string pack_model(const Model& m, const myo_task_cfg& cfg, PackedModel& out
   if (const char* ov = getenv("MYO_NLIM_CAP")) { const int v = atoi(ov); if (v >= 1 && v <= 32) nlim_fast = v; }
   B.finish();
   const int njmax = std::max(1, m.sz("njmax")), nconmax = std::max(1, m.sz("nconmax"));
-  auto layout = [&](DevModel& dd, int nlim_sides, int nlim_cap, int ncon_cap, int nefc_cap) {
+  // alias: the fast layout, which only the env step (and reset / get_obs, which run no physics) uses. Words of vectors
+  // whose lifetimes within a substep do not overlap are shared, so that more worlds fit an SM. The substep runs
+  //   tree_forward -> mass_bias -> tendon -> collision -> constraints -> actuation -> (qacc_smooth) -> solve -> integrate
+  // and the shared groups are
+  //   * solver vectors (solve .. integrate), observation (after the last substep), qfrc_bias (mass_bias .. actuation) and
+  //     ten_length / ten_velocity (tendon .. actuation);
+  //   * Newton Hessian (solve, and the M solves after actuation and in integrate) with xpos / xmat (tree_forward ..
+  //     collision, and the task's kinematics after the last substep), beside them the velocity-stage temporaries
+  //     (tree_forward .. mass_bias), the tendon phase's per-segment results and actuator force / qfrc_actuator /
+  //     qfrc_passive (actuation; never read after it).
+  // The full layout keeps every field in words of its own: the stage dumps of forward / mj_step read it.
+  auto layout = [&](DevModel& dd, bool alias, int nlim_sides, int nlim_cap, int ncon_cap, int nefc_cap) {
     dd.nlim_max = std::max(1, std::min(nlim * nlim_sides, nlim_cap));
     dd.ncon_max = std::max(1, std::min(dd.npair, ncon_cap));
     dd.nefc_max = std::min(dd.nlim_max + 4 * dd.ncon_max, nefc_cap);
@@ -586,47 +597,64 @@ std::string pack_model(const Model& m, const myo_task_cfg& cfg, PackedModel& out
     auto take = [&](int words) { int o = off; off += pad4(std::max(words, 1)); return o; };
     dd.o_qpos = take(nq); dd.o_qvel = take(nv); dd.o_act = take(na); dd.o_ctrl = take(nu); dd.o_warm = take(nv);
     dd.o_wparam = take(dd.nparam4);
-    dd.o_xpos = take(3 * nbody); dd.o_xmat = take(9 * nbody); dd.o_xipos = take(3 * nbody);
+    if (!alias) { dd.o_xpos = take(3 * nbody); dd.o_xmat = take(9 * nbody); }
+    dd.o_xipos = take(3 * nbody);
     dd.o_cdof = take(6 * nv);
     dd.o_M = take(nM);
-    dd.o_tenL = take(ntendon); dd.o_tenV = take(ntendon); dd.o_tenJ = take(ntendon * KT); dd.o_actF = take(nu);
-    dd.o_bias = take(nv); dd.o_passive = take(nv); dd.o_qact = take(nv); dd.o_smooth = take(nv); dd.o_qaccs = take(nv);
+    if (!alias) { dd.o_tenL = take(ntendon); dd.o_tenV = take(ntendon); }
+    dd.o_tenJ = take(ntendon * KT);
+    if (!alias) { dd.o_actF = take(nu); dd.o_bias = take(nv); dd.o_passive = take(nv); dd.o_qact = take(nv); }
+    dd.o_smooth = take(nv); dd.o_qaccs = take(nv);
     dd.o_qacc = take(nv); dd.o_qcon = take(nv); dd.o_actdot = take(na);
     // solver vectors; the observation (assembled after the last substep, when they are dead) shares their words
     {
       const int a0 = off;
       dd.o_grad = take(nv); dd.o_p = take(nv); dd.o_Mp = take(nv); dd.o_Ma = take(nv);
+      int words = off - a0;
+      if (alias) {
+        off = a0;
+        dd.o_bias = take(nv); dd.o_tenL = take(ntendon); dd.o_tenV = take(ntendon);
+        words = std::max(words, off - a0);
+      }
       dd.o_obs = a0;
-      off = a0 + std::max(off - a0, pad4(dd.nobs));
+      off = a0 + std::max(words, pad4(dd.nobs));
     }
     dd.o_misc = take(MI_WORDS);
     // velocity-stage temporaries and the composite inertias are dead once M and qfrc_bias exist; the Newton Hessian
     // (and the tendon phase's per-segment results) reuse their words
     {
       const int a0 = off;
-      dd.o_cdofdot = take(6 * nv); dd.o_cfrc = take(6 * nbody);
-      dd.o_cinert = take(10 * nbody);
-      const int tmp_words = off - a0;
       dd.o_H = a0;
       const int n4 = pad4(nv);
       int hw = 0;
       for (int i = 0; i < n4; i++) hw += 4 * ((i / 4 + 1) | 1);
       hw += n4;
-      off = a0 + std::max(tmp_words, hw);
+      if (alias) { dd.o_xpos = take(3 * nbody); dd.o_xmat = take(9 * nbody); }
+      const int a1 = off;      // from here on: words that are dead while the world's kinematics are live
+      dd.o_cdofdot = take(6 * nv); dd.o_cfrc = take(6 * nbody);
+      dd.o_cinert = take(10 * nbody);
+      int end = off;
+      if (alias) {
+        off = a1;
+        dd.o_actF = take(nu); dd.o_passive = take(nv); dd.o_qact = take(nv);
+        end = std::max(end, off);
+      }
+      dd.o_seg = a1;
+      off = std::max(end, a0 + hw);
       // limit / contact / row records follow directly: the tendon phase runs before they are rebuilt, so its per-segment
       // results may run on from the Hessian's words into theirs
       dd.o_lim = take(dd.nlim_max * LIM_WORDS); dd.o_con = take(dd.ncon_max * CON_WORDS); dd.o_row = take(dd.nefc_max * ROW_WORDS);
-      off = std::max(off, a0 + pad4(dd.nseg * SEG_OUT));
+      off = std::max(off, a1 + pad4(dd.nseg * SEG_OUT));
     }
     // world stride: tiles of one warp land on different banks
     if (out.lanes < 32) { while (off % 32 != out.lanes) off += 4; }
     else if (off % 32 == 0) off += 4;
     dd.scratch_words = off;
   };
-  layout(d, 1, nlim_fast, ncon_fast, nlim_fast + 4 * ncon_fast);
+  layout(d, true, 1, nlim_fast, ncon_fast, nlim_fast + 4 * ncon_fast);
   out.dm_full = d;
   // full capacities, bounded by what the solo kernel keeps in registers per lane (kSoloRowsPerLane rows)
-  layout(out.dm_full, 2, njmax, nconmax, std::min(njmax, kSoloRowsPerLane * out.lanes));
+  layout(out.dm_full, false, 2, njmax, nconmax, std::min(njmax, kSoloRowsPerLane * out.lanes));
   status = MYO_OK;
   return "";
 }

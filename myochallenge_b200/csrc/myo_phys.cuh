@@ -525,11 +525,12 @@ MYO_HELPER void segment_moment(int mslot, int soff, int list, const float* pa, c
 
 // One lane per path segment (results to scratch: length and moment-arm slots), then one lane per tendon adds its
 // segments in path order: ten_length, ten_J (KT slots over the tendon's dof list) and ten_velocity = J . qvel.
-// The per-segment results live in the Newton Hessian's scratch (free outside the constraint solve).
+// The per-segment results live in words the Newton Hessian and the records of the constraint phases use later
+// (myo_pack.cpp: o_seg).
 template <int G, int V>
 MYO_PHASE void phase_tendon(int mslot, Ctx<G, V> c, int* status) {
   MYO_M
-  float* res = SF(o_H);
+  float* res = SF(o_seg);
   for (int sg = c.lane; sg < m.nseg; sg += G) {
     const int* rec = m.seg_rec + sg * SEG_WORDS;
     const int type = rec[0] >> 16, id0 = rec[1], id1 = rec[2], g = rec[3], side = rec[4];
