@@ -11,10 +11,14 @@
  *                       (/root/reference/src/main_baoding.py:56-65,74) and the env kwargs of
  *                       /root/reference/src/envs/__init__.py:58-74 (Baoding P2), :137-150 (finger).
  *   myo_batch_reset  <- CustomBaodingP2Env.reset (/root/reference/src/envs/baoding.py:494-647),
- *                       CustomPoseEnv.reset (/root/reference/src/envs/pose.py:53-99).
+ *                       CustomPoseEnv.reset (/root/reference/src/envs/pose.py:53-99),
+ *                       MyoSuite 1.2.3 ReachEnvV0.reset, restated from memory ([3P-MEM], SURVEY.md), behind the
+ *                       factory names MyoFingerReachFixed / MyoFingerReachRandom
+ *                       (/root/reference/src/envs/environment_factory.py:22-61).
  *   myo_batch_step   <- VecEnv.step_async/step_wait -> env.step: BaodingEnvV1.step target update,
  *                       BaseV0.step action remap, Robot.step (frame_skip x mj_step), get_obs,
- *                       get_reward_dict (/root/reference/src/envs/baoding.py:403-467), TimeLimit and
+ *                       get_reward_dict (/root/reference/src/envs/baoding.py:403-467; reach: ReachEnvV0
+ *                       get_obs_dict / get_reward_dict [3P-MEM]), TimeLimit and
  *                       the SubprocVecEnv worker's auto-reset.
  *   myo_batch_mj_step / myo_batch_forward <- MjSim.step() / MjSim.forward()
  *                       (/root/reference/src/envs/baoding.py:183,206,625,632 reach them).
@@ -66,7 +70,7 @@ typedef enum {
   MYO_E_LIMIT = -6     /* model exceeds a compiled-in capacity */
 } myo_status;
 
-typedef enum { MYO_TASK_NONE = 0, MYO_TASK_POSE = 1, MYO_TASK_BAODING = 2, MYO_TASK_REORIENT = 3 } myo_task_kind;
+typedef enum { MYO_TASK_NONE = 0, MYO_TASK_POSE = 1, MYO_TASK_BAODING = 2, MYO_TASK_REORIENT = 3, MYO_TASK_REACH = 4 } myo_task_kind;
 
 /* Baoding `Task` enum values (MyoSuite baoding_v1.Task; 0 = hold, see
  * /root/reference/src/envs/baoding.py:287-294, /root/reference/src/models/classifier.py:116) */
@@ -100,7 +104,8 @@ typedef struct myo_task_cfg {
   /* reward weights, in the order written to info[] (slot 7 always carries the dense reward):
    *  baoding : pos_dist_1 pos_dist_2 act_reg alive sparse solved done dense
    *  pose    : pose bonus penalty act_reg sparse solved done dense
-   *  reorient: pos_dist rot_dist act_reg alive sparse solved done dense pos_dist_diff rot_dist_diff */
+   *  reorient: pos_dist rot_dist act_reg alive sparse solved done dense pos_dist_diff rot_dist_diff
+   *  reach   : reach bonus act_reg penalty sparse solved done dense */
   float rwd_weight[MYO_INFO_TERMS];
   /* ---- baoding ---- */
   float drop_th, proximity_th;
@@ -115,14 +120,14 @@ typedef struct myo_task_cfg {
   int32_t ball_body[2], ball_geom[2], ball_site[2], target_site[2];
   int32_t ball_qposadr[2], ball_dofadr[2];
   /* ---- pose ---- */
-  float pose_thd, far_th, target_distance;
+  float pose_thd, far_th, target_distance;   /* reach: far_th is the whole threshold, ReachEnvV0's far_th x reach_nsite */
   int32_t reset_type;           /* 0 none, 1 init, 2 random, 3 sds */
   int32_t target_type;          /* 0 fixed, 1 generate */
   int32_t n_target_jnt;         /* <=0: target_jnt_value given for all nq */
   int32_t target_jnt_ids[64];
   float target_jnt_range[64][2];
   float target_jnt_value[64];
-  /* ---- overrides (filled by the library for baoding; free for other tasks) ---- */
+  /* ---- overrides (filled by the library for baoding; free for other tasks; reach ignores ovr_site and uses its target sites) ---- */
   int32_t n_ovr_body, ovr_body[MYO_MAX_OVERRIDE];
   int32_t n_ovr_geom, ovr_geom[MYO_MAX_OVERRIDE];
   int32_t n_ovr_site, ovr_site[MYO_MAX_OVERRIDE];
@@ -156,6 +161,15 @@ typedef struct myo_task_cfg {
   int32_t weight_body;          /* >= 0: body_mass[weight_body] ~ U(weight_range) per reset, geom_size[weight_geom][0] = 0.01 + 2.5 w / 100 */
   int32_t weight_geom;
   float weight_range[2];
+  /* ---- reach: MyoSuite ReachEnvV0 (envs/myo/reach_v0.py). Each tip site has a target site ("<tip>_target") whose site_pos
+   *      reset() draws uniformly inside (low, high); the targets are per-world MYO_PARAM_SITE_POS overrides. ---- */
+  int32_t reach_nsite;                          /* 1 .. MYO_MAX_OVERRIDE (more: MYO_E_LIMIT) */
+  int32_t reach_tip_site[MYO_MAX_OVERRIDE], reach_target_site[MYO_MAX_OVERRIDE];
+  float reach_range[MYO_MAX_OVERRIDE][2][3];    /* [site][low, high][x, y, z] of the target's site_pos */
+  float reach_near_th;                          /* 0.0125 x reach_nsite: bonus below 2 near_th and near_th, solved below near_th */
+  int32_t reach_far_steps;                      /* far_th applies from this many elapsed env steps on: ReachEnvV0 compares
+                                                   data.time > 2 dt, with time summed in fp64 once per substep (myosuite keeps
+                                                   far_th = inf before), so the first such step count is worked out on the host */
 } myo_task_cfg;
 
 const char* myo_last_error(void);

@@ -15,7 +15,7 @@ MYO_MAX_OVERRIDE = 4
 MYO_INFO_TERMS = 12
 MYO_MAX_ROT_RANGES = 4
 TASK_STATE_I, TASK_STATE_F = 4, 8
-TASK_NONE, TASK_POSE, TASK_BAODING, TASK_REORIENT = 0, 1, 2, 3
+TASK_NONE, TASK_POSE, TASK_BAODING, TASK_REORIENT, TASK_REACH = 0, 1, 2, 3, 4
 PARAM_BODY_MASS, PARAM_GEOM_SIZE, PARAM_GEOM_FRICTION, PARAM_SITE_POS, PARAM_BODY_POS, PARAM_BODY_MAT = 0, 1, 2, 3, 4, 5
 PARAM_NCOMP = {0: 1, 1: 3, 2: 3, 3: 3, 4: 3, 5: 9}
 
@@ -61,6 +61,8 @@ class TaskCfg(C.Structure):
         ("goal_init_pos", C.c_float * 3), ("goal_obj_offset", C.c_float * 3),
         ("n_ovr_bodypose", C.c_int32), ("ovr_bodypose", C.c_int32 * MYO_MAX_OVERRIDE),
         ("sds_distance", C.c_float), ("weight_body", C.c_int32), ("weight_geom", C.c_int32), ("weight_range", C.c_float * 2),
+        ("reach_nsite", C.c_int32), ("reach_tip_site", C.c_int32 * MYO_MAX_OVERRIDE), ("reach_target_site", C.c_int32 * MYO_MAX_OVERRIDE),
+        ("reach_range", ((C.c_float * 3) * 2) * MYO_MAX_OVERRIDE), ("reach_near_th", C.c_float), ("reach_far_steps", C.c_int32),
     ]
 
 

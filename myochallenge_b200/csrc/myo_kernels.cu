@@ -120,7 +120,7 @@ __device__ void run_world(int mslot, const myo_task_cfg& t, const BatchPtrs& b, 
     task_obs<G>(mslot, t, c, ptarget);
     float info[MYO_INFO_TERMS], reward;
     bool env_done;
-    task_reward<G>(mslot, t, c, tf, info, &reward, &env_done);
+    task_reward<G>(mslot, t, c, tf, ti[TI_ELAPSED] + 1, info, &reward, &env_done);
     // a world whose state left the finite range ends its episode here (MuJoCo would warn and reset the data): the reset
     // below keeps NaNs out of the running moments downstream
     bool bad = false;
@@ -692,6 +692,24 @@ int myo_task_cfg_default(const myo_model* mh, int kind, myo_task_cfg* cfg) {
     cfg->pose_thd = 0.35f; cfg->far_th = 4.f * 3.14159265358979f / 2.f; cfg->target_distance = 1.f;
     cfg->reset_type = 1; cfg->target_type = 1;
     cfg->weight_body = -1; cfg->weight_geom = -1;
+  } else if (kind == MYO_TASK_REACH) {
+    // ReachEnvV0._setup defaults (far_th .35, reach 1 / bonus 4 / penalty 50) and the myoFingerReach* registrations (frame_skip 5,
+    // 200 steps), MyoSuite 1.2.3 [3P-MEM]. Sites: IFtip when the model has it, its target held at the model's site_pos.
+    cfg->frame_skip = 5; cfg->max_episode_steps = 200;
+    cfg->rwd_weight[0] = 1.f; cfg->rwd_weight[1] = 4.f; cfg->rwd_weight[3] = 50.f;
+    const int tip = m.name2id("site", "IFtip"), tgt = m.name2id("site", "IFtip_target");
+    if (tip >= 0 && tgt >= 0) {
+      cfg->reach_nsite = 1; cfg->reach_tip_site[0] = tip; cfg->reach_target_site[0] = tgt;
+      const double* sp = m.d("site_pos") + 3 * tgt;
+      for (int e = 0; e < 3; e++) cfg->reach_range[0][0][e] = cfg->reach_range[0][1][e] = (float)sp[e];
+    }
+    cfg->far_th = 0.35f; cfg->reach_near_th = 0.0125f;
+    // first env step after which time > 2 dt, with time summed in fp64 one substep at a time as MuJoCo does
+    const double h = m.opt.at("timestep"), dt = h * cfg->frame_skip;
+    double time = 0.0;
+    int k = 0;
+    while (!(time > 2.0 * dt)) { for (int s = 0; s < cfg->frame_skip; s++) time += h; k++; }
+    cfg->reach_far_steps = k;
   }
   return MYO_OK;
 }
@@ -706,6 +724,14 @@ int myo_model_check(const myo_model* mh, char* report, size_t report_len) {
 
 int myo_batch_create(const myo_model* mh, int n_worlds, int device, const myo_task_cfg* cfg, uint64_t seed, myo_batch** out) {
   if (!mh || !cfg || !out || n_worlds <= 0) { myo::set_error("bad argument to myo_batch_create"); return MYO_E_ARG; }
+  if (cfg->kind == MYO_TASK_REACH) {
+    if (cfg->reach_nsite > MYO_MAX_OVERRIDE) { myo::set_error("reach: more target sites than MYO_MAX_OVERRIDE"); return MYO_E_LIMIT; }
+    const int nsite = myo_model_host(mh).sz("nsite");
+    bool ok = cfg->reach_nsite >= 1;
+    for (int k = 0; ok && k < cfg->reach_nsite; k++)
+      ok = cfg->reach_tip_site[k] >= 0 && cfg->reach_tip_site[k] < nsite && cfg->reach_target_site[k] >= 0 && cfg->reach_target_site[k] < nsite;
+    if (!ok) { myo::set_error("reach: needs 1..MYO_MAX_OVERRIDE tip / target sites with valid ids"); return MYO_E_ARG; }
+  }
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0 || device < 0 || device >= ndev) {
     myo::set_error("no CUDA device available (this library has no CPU path)");

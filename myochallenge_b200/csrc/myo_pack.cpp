@@ -202,8 +202,10 @@ std::string pack_model(const Model& m, const myo_task_cfg& cfg, PackedModel& out
       for (int e = 0; e < 3; e++) out.param0.push_back((float)gf[3 * g + e]);
       np += 3;
     }
-    for (int k = 0; k < cfg.n_ovr_site && k < MYO_MAX_OVERRIDE; k++) {
-      int s = cfg.ovr_site[k];
+    // reach: the target sites are the per-world site overrides (reset draws them)
+    const bool reach = cfg.kind == MYO_TASK_REACH;
+    for (int k = 0; k < (reach ? cfg.reach_nsite : cfg.n_ovr_site) && k < MYO_MAX_OVERRIDE; k++) {
+      int s = reach ? cfg.reach_target_site[k] : cfg.ovr_site[k];
       if (s < 0 || s >= nsite) { status = MYO_E_ARG; return "override site id out of range"; }
       spos_slot[s] = np; out.slots.push_back({MYO_PARAM_SITE_POS, s, np, 3});
       for (int e = 0; e < 3; e++) out.param0.push_back((float)sp[3 * s + e]);
@@ -524,6 +526,7 @@ std::string pack_model(const Model& m, const myo_task_cfg& cfg, PackedModel& out
   if (cfg.kind == MYO_TASK_BAODING) d.nobs = (nq - 14) + 24 + na;
   else if (cfg.kind == MYO_TASK_POSE) d.nobs = nq + nv + nq + na;
   else if (cfg.kind == MYO_TASK_REORIENT) d.nobs = (nq - 7) + (nv - 6) + 18 + na;
+  else if (cfg.kind == MYO_TASK_REACH) d.nobs = nq + nv + 6 * cfg.reach_nsite + na;      // qpos qvel*dt tip_pos reach_err act
   else d.nobs = nq + nv + na;
   d.nobs4 = pad4(d.nobs);
   {

@@ -4,7 +4,9 @@
 //            /root/reference/src/envs/baoding.py:186-190,627-631 (SURVEY.md 8a row a11)
 //   pose   : CustomPoseEnv.reset / get_target_pose (/root/reference/src/envs/pose.py:53-113) on
 //            MyoSuite PoseEnvV0 obs / reward keys
-//   both   : BaseV0.step muscle action remap, gym TimeLimit, SubprocVecEnv worker auto-reset.
+//   reach  : MyoSuite 1.2.3 ReachEnvV0 get_obs_dict / get_reward_dict / generate_target_pose + reset, restated from memory
+//            ([3P-MEM], SURVEY.md) behind MyoFingerReachFixed / MyoFingerReachRandom (/root/reference/src/envs/environment_factory.py)
+//   all    : BaseV0.step muscle action remap, gym TimeLimit, SubprocVecEnv worker auto-reset.
 #pragma once
 #include "myo_phys.cuh"
 
@@ -131,6 +133,19 @@ MYO_PHASE void task_obs(int mslot, const myo_task_cfg& t, Ctx<G, V> c, const flo
         obs[o0 + 9 + e] = eo[e]; obs[o0 + 12 + e] = eg[e]; obs[o0 + 15 + e] = eg[e] - eo[e];
       }
     }
+  } else if (t.kind == MYO_TASK_REACH) {
+    // ReachEnvV0.get_obs_dict: qpos | qvel * dt | tip_pos | reach_err = target_pos - tip_pos | act, sites in target_reach_range order
+    const int o0 = m.nq + m.nv, ns = t.reach_nsite;
+    for (int i = c.lane; i < m.nq; i += G) obs[i] = qpos[i];
+    for (int i = c.lane; i < m.nv; i += G) obs[m.nq + i] = qvel[i] * m.frame_dt;
+    for (int i = c.lane; i < m.na; i += G) obs[o0 + 6 * ns + i] = act[i];
+    for (int k = c.lane; k < ns; k += G) {
+      float p[3], g[3];
+      site_world(m, c.sp(), c.wpp(m), t.reach_tip_site[k], p);
+      site_world(m, c.sp(), c.wpp(m), t.reach_target_site[k], g);
+#pragma unroll
+      for (int e = 0; e < 3; e++) { obs[o0 + 3 * k + e] = p[e]; obs[o0 + 3 * ns + 3 * k + e] = g[e] - p[e]; }
+    }
   } else {
     for (int i = c.lane; i < m.nq; i += G) obs[i] = qpos[i];
     for (int i = c.lane; i < m.nv; i += G) obs[m.nq + i] = qvel[i];
@@ -139,10 +154,41 @@ MYO_PHASE void task_obs(int mslot, const myo_task_cfg& t, Ctx<G, V> c, const flo
   c.tile.sync();
 }
 
-// reward terms + dense reward + termination from the observation in scratch. info: MYO_INFO_TERMS floats.
+// ReachEnvV0.get_reward_dict from the observation in scratch: one distance over all 3 n entries of reach_err. ReachEnvV0 applies
+// far_th only once data.time > 2 dt; `elapsed` (env steps since the reset, this one included) stands in for the time.
 template <int G, int V>
-MYO_PHASE void task_reward(int mslot, const myo_task_cfg& t, Ctx<G, V> c, float* tf, float* info, float* reward, bool* done) {
+MYO_PHASE void reach_reward(int mslot, const myo_task_cfg& t, Ctx<G, V> c, int elapsed, float* info, float* reward, bool* done) {
   MYO_M
+  const float* obs = SF(o_obs); const float* act = SF(o_act);
+  float a2 = 0.f;
+  for (int i = c.lane; i < m.na; i += G) a2 += act[i] * act[i];
+  a2 = tile_sum<G>(c, a2);
+  const float act_mag = m.na ? sqrtf(a2) / (float)m.na : 0.f;
+  const float* err = obs + m.nq + m.nv + 3 * t.reach_nsite;
+  float e2 = 0.f;
+  for (int i = 0; i < 3 * t.reach_nsite; i++) e2 += err[i] * err[i];
+  const float d = sqrtf(e2), near = t.reach_near_th;
+  const bool far = elapsed >= t.reach_far_steps && d > t.far_th;
+  float term[MYO_INFO_TERMS];
+#pragma unroll
+  for (int k = 0; k < MYO_INFO_TERMS; k++) term[k] = 0.f;
+  term[0] = -d; term[1] = (d < 2.f * near ? 1.f : 0.f) + (d < near ? 1.f : 0.f); term[2] = -act_mag;
+  term[3] = far ? -1.f : 0.f; term[4] = -d; term[5] = d < near ? 1.f : 0.f; term[6] = far ? 1.f : 0.f;
+  float dense = 0.f;
+#pragma unroll
+  for (int k = 0; k < MYO_INFO_TERMS; k++) if (k != 7) dense += t.rwd_weight[k] * term[k];
+  term[7] = dense;
+#pragma unroll
+  for (int k = 0; k < MYO_INFO_TERMS; k++) info[k] = term[k];
+  *reward = dense; *done = far;
+}
+
+// reward terms + dense reward + termination from the observation in scratch. info: MYO_INFO_TERMS floats. elapsed: env steps
+// since the reset, this one included.
+template <int G, int V>
+MYO_PHASE void task_reward(int mslot, const myo_task_cfg& t, Ctx<G, V> c, float* tf, int elapsed, float* info, float* reward, bool* done) {
+  MYO_M
+  if (t.kind == MYO_TASK_REACH) { reach_reward<G>(mslot, t, c, elapsed, info, reward, done); return; }
   const float* obs = SF(o_obs); const float* act = SF(o_act);
   float a2 = 0.f;
   for (int i = c.lane; i < m.na; i += G) a2 += act[i] * act[i];
@@ -387,6 +433,15 @@ MYO_PHASE void task_reset(int mslot, const myo_task_cfg& t, Ctx<G, V> c, const B
         for (int j = 0; j < m.njnt; j++)
           if (m.j_type[j] == J_HINGE || m.j_type[j] == J_SLIDE)
             qpos[m.j_qposadr[j]] = rng.uniform(m.j_range[2 * j], m.j_range[2 * j + 1]);
+      }
+    } else if (t.kind == MYO_TASK_REACH) {
+      // ReachEnvV0.generate_target_pose: site_pos[<tip>_target] = np_random.uniform(low, high), x y z of each site in turn
+      for (int k = 0; k < t.reach_nsite; k++) {
+        const int slot = m.s_pos_slot[t.reach_target_site[k]];
+        for (int e = 0; e < 3; e++) {
+          const float v = rng.uniform(t.reach_range[k][0][e], t.reach_range[k][1][e]);
+          if (slot >= 0) c.wpp(m)[slot + e] = v;
+        }
       }
     }
   }

@@ -18,7 +18,7 @@ import numpy as np
 from . import _capi
 from .assets import asset_path
 from .sim import Model
-from .vec_env import BAODING_KEYS, POSE_KEYS, REORIENT_KEYS, MyoVecEnv
+from .vec_env import BAODING_KEYS, POSE_KEYS, REACH_KEYS, REORIENT_KEYS, MyoVecEnv
 
 _JNT_HAND = ['pro_sup', 'deviation', 'flexion', 'cmc_abduction', 'cmc_flexion', 'mp_flexion', 'ip_flexion', 'mcp2_flexion',
              'mcp2_abduction', 'pm2_flexion', 'md2_flexion', 'mcp3_flexion', 'mcp3_abduction', 'pm3_flexion', 'md3_flexion',
@@ -82,6 +82,15 @@ REGISTRY["myoChallengeBaodingP2-v1"] = REGISTRY["CustomMyoChallengeBaodingP2-v1"
 REGISTRY["myoChallengeBaodingP1-v1"] = REGISTRY["CustomMyoChallengeBaodingP1-v1"]
 REGISTRY["myoHandPoseRandom-v0"] = REGISTRY["CustomMyoHandPoseRandom-v0"]
 REGISTRY["myoElbowPose1D6MRandom-v0"] = REGISTRY["CustomMyoElbowPoseRandom-v0"]
+# MyoSuite 1.2.3 envs/myo/__init__.py finger reach registrations (ReachEnvV0), as best recalled [3P-MEM]. The Random range has
+# one check: at the model's qpos0 the oracle puts IFtip at (0.270, 0.000, 0.300), that range's upper corner. The frame skip and
+# the horizon have no such check.
+REGISTRY["myoFingerReachFixed-v0"] = dict(kind=_capi.TASK_REACH, model="finger/myo_finger_v0.mjb", horizon=200,
+                                          kwargs=dict(target_reach_range={"IFtip": ((0.2, 0.05, 0.20), (0.2, 0.05, 0.20))},
+                                                      normalize_act=True, frame_skip=5))
+REGISTRY["myoFingerReachRandom-v0"] = dict(kind=_capi.TASK_REACH, model="finger/myo_finger_v0.mjb", horizon=200,
+                                           kwargs=dict(target_reach_range={"IFtip": ((.1, -.1, .1), (.27, .1, .3))},
+                                                       normalize_act=True, frame_skip=5))
 
 # EnvironmentFactory names -> gym ids   [REF src/envs/environment_factory.py:22-61]
 FACTORY_NAMES = {
@@ -92,10 +101,21 @@ FACTORY_NAMES = {
     "CustomMyoFingerPoseFixed": "CustomMyoFingerPoseFixed-v0", "CustomMyoFingerPoseRandom": "CustomMyoFingerPoseRandom-v0",
     "CustomMyoHandPoseFixed": "CustomMyoHandPoseFixed-v0", "CustomMyoHandPoseRandom": "CustomMyoHandPoseRandom-v0",
     "CustomMyoReorientP1": "CustomMyoChallengeDieReorientP1-v0", "CustomMyoReorientP2": "CustomMyoChallengeDieReorientP2-v0",
+    "MyoFingerReachFixed": "myoFingerReachFixed-v0", "MyoFingerReachRandom": "myoFingerReachRandom-v0",
 }
-# names the reference factory knows whose models / task kernels are outside this build (pen, key-turn, reach, mixture)
-UNSUPPORTED = {"MyoFingerReachFixed", "MyoFingerReachRandom", "MyoHandKeyTurnFixed", "MyoHandKeyTurnRandom",
-               "MixtureModelBaodingEnv", "CustomMyoPenTwirlRandom"}
+# names the reference factory knows whose models / task kernels are outside this build (pen, key-turn, mixture)
+UNSUPPORTED = {"MyoHandKeyTurnFixed", "MyoHandKeyTurnRandom", "MixtureModelBaodingEnv", "CustomMyoPenTwirlRandom"}
+
+
+def reach_far_steps(timestep: float, frame_skip: int) -> int:
+    """First env step count after which ReachEnvV0 applies far_th (``data.time > 2 dt``): MuJoCo adds ``timestep`` to ``time``
+    in fp64 once per substep, so the sum is replayed here (the kernel keeps time in fp32 and compares step counts instead)."""
+    dt, t, k = timestep * frame_skip, 0.0, 0
+    while not t > 2 * dt:
+        for _ in range(frame_skip):
+            t += timestep
+        k += 1
+    return k
 
 
 def _weights(cfg, keys, weighted_reward_keys):
@@ -189,6 +209,25 @@ def make_task_cfg(model: Model, env_id: str, **overrides) -> _capi.TaskCfg:
         # MuJoCo's kinematics never reads (a free body's pose is its qpos), so these knobs change nothing there - nor here
         for k in ("enable_rsi", "rsi_distance_pos", "rsi_distance_rot"):
             kw.pop(k, None)
+    elif reg["kind"] == _capi.TASK_REACH:
+        # ReachEnvV0._setup(target_reach_range, far_th=.35, ...) [3P-MEM]: thresholds scale with the number of sites
+        if "weighted_reward_keys" in kw:
+            _weights(cfg, REACH_KEYS, kw.pop("weighted_reward_keys"))
+        sites = dict(kw.pop("target_reach_range"))
+        if not 0 < len(sites) <= _capi.MYO_MAX_OVERRIDE:
+            raise ValueError(f"target_reach_range: between 1 and {_capi.MYO_MAX_OVERRIDE} sites (the targets use the per-world site overrides)")
+        cfg.reach_nsite = len(sites)
+        for k, (site, (lo, hi)) in enumerate(sites.items()):
+            try:
+                cfg.reach_tip_site[k], cfg.reach_target_site[k] = model.name2id("site", site), model.name2id("site", site + "_target")
+            except KeyError:
+                raise ValueError(f"target_reach_range: the model has no sites {site!r} and {site + '_target'!r}") from None
+            lo, hi = np.asarray(lo, float).reshape(3), np.asarray(hi, float).reshape(3)
+            for e in range(3):
+                cfg.reach_range[k][0][e], cfg.reach_range[k][1][e] = lo[e], hi[e]
+        cfg.far_th = float(kw.pop("far_th", 0.35)) * len(sites)
+        cfg.reach_near_th = 0.0125 * len(sites)
+        cfg.reach_far_steps = reach_far_steps(model.opt("timestep"), cfg.frame_skip)
     else:
         if "weighted_reward_keys" in kw:
             _weights(cfg, POSE_KEYS, kw.pop("weighted_reward_keys"))

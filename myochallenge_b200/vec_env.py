@@ -75,6 +75,8 @@ BAODING_KEYS = ("pos_dist_1", "pos_dist_2", "act_reg", "alive", "sparse", "solve
 POSE_KEYS = ("pose", "bonus", "penalty", "act_reg", "sparse", "solved", "done")
 # CustomReorientEnv.get_reward_dict (/root/reference/src/envs/reorient.py:21-46); slot 7 is the dense reward in every task
 REORIENT_KEYS = ("pos_dist", "rot_dist", "act_reg", "alive", "sparse", "solved", "done", "dense", "pos_dist_diff", "rot_dist_diff")
+# MyoSuite ReachEnvV0.get_reward_dict [3P-MEM]
+REACH_KEYS = ("reach", "bonus", "act_reg", "penalty", "sparse", "solved", "done")
 
 
 class MyoVecEnv:
@@ -87,7 +89,11 @@ class MyoVecEnv:
         self.cfg = cfg
         self.observation_space = Box(-10.0, 10.0, (self.sim.nobs,), np.float32)
         self.action_space = Box(-1.0, 1.0, (self.sim.nu,), np.float32)
-        self._keys = {_capi.TASK_BAODING: BAODING_KEYS, _capi.TASK_REORIENT: REORIENT_KEYS}.get(cfg.kind, POSE_KEYS)
+        keys = {_capi.TASK_BAODING: BAODING_KEYS, _capi.TASK_REORIENT: REORIENT_KEYS, _capi.TASK_REACH: REACH_KEYS,
+                _capi.TASK_POSE: POSE_KEYS, _capi.TASK_NONE: POSE_KEYS}
+        if cfg.kind not in keys:
+            raise ValueError(f"no reward keys for task kind {cfg.kind}")
+        self._keys = keys[cfg.kind]
         self.info_keys = tuple(self._keys)      # names of the columns of ``sim.info`` (the reward terms ``infos[i]`` carries)
         n, pin = self.num_envs, self.device.type == "cuda"
         self._h_act = torch.zeros(n, self.sim.nu, dtype=torch.float32, pin_memory=pin)

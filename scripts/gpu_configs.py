@@ -9,7 +9,7 @@ from myochallenge_b200.policy import RecurrentPolicy
 dev = "cuda:0"
 for env_id, n in (("CustomMyoElbowPoseRandom-v0", 1), ("CustomMyoElbowPoseRandom-v0", 65536), ("CustomMyoFingerPoseRandom-v0", 4096),
                   ("CustomMyoFingerPoseRandom-v0", 65536), ("CustomMyoHandPoseRandom-v0", 16384), ("CustomMyoChallengeDieReorientP2-v0", 16384),
-                  ("CustomMyoChallengeBaodingP1-v1", 32768)):
+                  ("CustomMyoChallengeBaodingP1-v1", 32768), ("myoFingerReachRandom-v0", 4096), ("myoFingerReachRandom-v0", 65536)):
     env = make_vec_env(env_id, n, device=dev, seed=0, clip_actions=True)
     pol = RecurrentPolicy(env.sim.nobs, env.sim.nu, 256, (256, 256), (256, 256), max_batch=n, device=dev)
     pol.init_random(0, -2.0); pol.seed(1)
