@@ -89,6 +89,22 @@ typedef enum {
 #define MYO_MAX_OVERRIDE 4
 #define MYO_INFO_TERMS 12
 #define MYO_MAX_ROT_RANGES 4
+#define MYO_MAX_OBS_KEYS 16
+
+/* Observation keys (MyoSuite's obs_keys): ids of the obs-dict entries of each task kind, numbered in the order of its
+ * get_obs_dict. myo_task_cfg.obs_keys lists them in the order they are concatenated; duplicates are allowed. The ids of a
+ * key list are those of cfg.kind. */
+enum { MYO_OBS_BAODING_T = 0, MYO_OBS_BAODING_HAND_POS = 1, MYO_OBS_BAODING_OBJECT1_POS = 2, MYO_OBS_BAODING_OBJECT1_VELP = 3,
+       MYO_OBS_BAODING_OBJECT2_POS = 4, MYO_OBS_BAODING_OBJECT2_VELP = 5, MYO_OBS_BAODING_TARGET1_POS = 6,
+       MYO_OBS_BAODING_TARGET2_POS = 7, MYO_OBS_BAODING_TARGET1_ERR = 8, MYO_OBS_BAODING_TARGET2_ERR = 9, MYO_OBS_BAODING_ACT = 10,
+       MYO_OBS_BAODING_COUNT = 11 };
+enum { MYO_OBS_REORIENT_T = 0, MYO_OBS_REORIENT_HAND_QPOS = 1, MYO_OBS_REORIENT_HAND_QVEL = 2, MYO_OBS_REORIENT_OBJ_POS = 3,
+       MYO_OBS_REORIENT_GOAL_POS = 4, MYO_OBS_REORIENT_POS_ERR = 5, MYO_OBS_REORIENT_OBJ_ROT = 6, MYO_OBS_REORIENT_GOAL_ROT = 7,
+       MYO_OBS_REORIENT_ROT_ERR = 8, MYO_OBS_REORIENT_ACT = 9, MYO_OBS_REORIENT_COUNT = 10 };
+enum { MYO_OBS_POSE_T = 0, MYO_OBS_POSE_QPOS = 1, MYO_OBS_POSE_QVEL = 2, MYO_OBS_POSE_ACT = 3, MYO_OBS_POSE_POSE_ERR = 4,
+       MYO_OBS_POSE_COUNT = 5 };
+enum { MYO_OBS_REACH_T = 0, MYO_OBS_REACH_QPOS = 1, MYO_OBS_REACH_QVEL = 2, MYO_OBS_REACH_ACT = 3, MYO_OBS_REACH_TIP_POS = 4,
+       MYO_OBS_REACH_TARGET_POS = 5, MYO_OBS_REACH_REACH_ERR = 6, MYO_OBS_REACH_COUNT = 7 };
 
 /* Task / env configuration: the kwargs of the gym registrations plus the curriculum knobs of
  * CustomBaodingP2Env._setup (/root/reference/src/envs/baoding.py:300-401) and
@@ -170,6 +186,16 @@ typedef struct myo_task_cfg {
   int32_t reach_far_steps;                      /* far_th applies from this many elapsed env steps on: ReachEnvV0 compares
                                                    data.time > 2 dt, with time summed in fp64 once per substep (myosuite keeps
                                                    far_th = inf before), so the first such step count is worked out on the host */
+  /* ---- observation layout and reward mode: MyoSuite's obs_keys / reward_mode kwargs (MujocoEnv._setup) ---- */
+  int32_t n_obs_keys;                           /* 0: the kind's default layout (below); 1 .. MYO_MAX_OBS_KEYS (more: MYO_E_LIMIT) */
+  int32_t obs_keys[MYO_MAX_OBS_KEYS];           /* MYO_OBS_<KIND>_* ids, concatenated in this order. Default layouts:
+                                                   baoding : hand_pos object1_pos object1_velp object2_pos object2_velp target1_pos
+                                                             target2_pos target1_err target2_err act
+                                                   reorient: hand_qpos hand_qvel obj_pos goal_pos pos_err obj_rot goal_rot rot_err act
+                                                   pose    : qpos qvel pose_err act
+                                                   reach   : qpos qvel tip_pos reach_err act
+                                                   t is the world's time after the step (0 right after a reset) */
+  int32_t reward_sparse;                        /* 1: the step's reward is info[4] (the sparse term of every kind), 0: the dense reward */
 } myo_task_cfg;
 
 const char* myo_last_error(void);
@@ -226,7 +252,8 @@ int myo_batch_get_param(myo_batch* b, int kind, int id, float* values_dev, void*
 #define MYO_TASK_STATE_F 8
 int myo_batch_get_task_state(myo_batch* b, int32_t* ti_dev, float* tf_dev, float* pose_target_dev, void* stream);
 int myo_batch_set_task_state(myo_batch* b, const int32_t* ti_dev, const float* tf_dev, const float* pose_target_dev, void* stream);
-/* one env step for every world. actions[n,nu] in [-1,1]; obs[n,nobs]; reward[n]; done[n] (env
+/* one env step for every world. actions[n,nu] in [-1,1]; obs[n,nobs] (nobs: myo_batch_dims, the width of the cfg's obs_keys);
+ * reward[n] (dense, or info[4] with reward_sparse); done[n] (env
  * termination OR time limit, as SB3 sees it); truncated[n] (TimeLimit.truncated);
  * terminal_obs[n,nobs] (written for worlds that finished; may be NULL); info[n,MYO_INFO_TERMS]
  * reward terms + dense (may be NULL). */

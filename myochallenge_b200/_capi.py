@@ -14,6 +14,7 @@ LIB_PATH = os.path.join(_HERE, "libmyo_b200.so")
 MYO_MAX_OVERRIDE = 4
 MYO_INFO_TERMS = 12
 MYO_MAX_ROT_RANGES = 4
+MYO_MAX_OBS_KEYS = 16
 TASK_STATE_I, TASK_STATE_F = 4, 8
 TASK_NONE, TASK_POSE, TASK_BAODING, TASK_REORIENT, TASK_REACH = 0, 1, 2, 3, 4
 PARAM_BODY_MASS, PARAM_GEOM_SIZE, PARAM_GEOM_FRICTION, PARAM_SITE_POS, PARAM_BODY_POS, PARAM_BODY_MAT = 0, 1, 2, 3, 4, 5
@@ -63,6 +64,7 @@ class TaskCfg(C.Structure):
         ("sds_distance", C.c_float), ("weight_body", C.c_int32), ("weight_geom", C.c_int32), ("weight_range", C.c_float * 2),
         ("reach_nsite", C.c_int32), ("reach_tip_site", C.c_int32 * MYO_MAX_OVERRIDE), ("reach_target_site", C.c_int32 * MYO_MAX_OVERRIDE),
         ("reach_range", ((C.c_float * 3) * 2) * MYO_MAX_OVERRIDE), ("reach_near_th", C.c_float), ("reach_far_steps", C.c_int32),
+        ("n_obs_keys", C.c_int32), ("obs_keys", C.c_int32 * MYO_MAX_OBS_KEYS), ("reward_sparse", C.c_int32),
     ]
 
 

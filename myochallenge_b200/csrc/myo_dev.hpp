@@ -68,6 +68,10 @@ struct DevModel {
   // sizes
   int nq, nv, nu, na, nbody, njnt, ngeom, nsite, ntendon, nwrap, nM, npair, nlevel, ndlevel;
   int nq4, nv4, na4, nu4, nparam, nparam4, nobs, nobs4;
+  // observation: task_obs writes the kind's canonical layout (nobs_scr words at o_obs), the caller's buffers take nobs words.
+  // With obs_keys the output is gathered from nobs_run runs: obs_run[r] = source word | width << 16 | OBS_RUN_* << 28
+  // (nobs_run 0: the canonical layout as it is, nobs == nobs_scr)
+  int nobs_scr, nobs_run, obs_run[MYO_MAX_OBS_KEYS];
   int nlim_max, ncon_max, nefc_max;
   int nd;   // dofs [0, nd) couple through the mass matrix; dofs [nd, nv) are simple (diagonal)
   TabI pair_ab;  // unordered support pairs of a contact block (myo_pack.cpp)
@@ -152,6 +156,8 @@ enum { TI_ELAPSED = 0, TI_EPISODE = 1, TI_TASK = 2, TI_FLAGS = 3, TI_WORDS = 4 }
 enum { TF_ANGLE1 = 0, TF_ANGLE2 = 1, TF_XR = 2, TF_YR = 3, TF_PERIOD = 4, TF_POSDIST = 5, TF_ROTDIST = 6, TF_WORDS = 8 };
 // o_misc scratch words
 enum { MI_NLIM = 0, MI_NCON = 1, MI_NEFC = 2, MI_ITER = 3, MI_STATUS = 4, MI_ONE = 5 /*float 1*/, MI_WORDS = 8 };
+
+enum { OBS_RUN_COPY = 0, OBS_RUN_TIME = 1 /* the world's time, width 1 */, OBS_RUN_SUM = 2 /* src[i] + src[width + i] */ };
 
 enum StepMode { MODE_ENV_STEP = 0, MODE_MJ_STEP = 1, MODE_FORWARD = 2, MODE_GET_OBS = 3, MODE_RESET = 4, MODE_REDO = 5 };
 enum { REDO_STEP = 0, REDO_RESET = 1 };      // kinds of redo-list entries

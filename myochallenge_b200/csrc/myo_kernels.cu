@@ -78,7 +78,7 @@ __device__ void run_world(int mslot, const myo_task_cfg& t, const BatchPtrs& b, 
     if (a.obs && io) {
       phase_tree_forward<G>(mslot, c, false);
       task_obs<G>(mslot, t, c, ptarget);
-      for (int i = c.lane; i < m.nobs; i += G) a.obs[(size_t)w * m.nobs + i] = SF(o_obs)[i];
+      write_obs<G>(mslot, c, a.obs + (size_t)w * m.nobs, b.time + w, false);
     }
     store_world<G>(mslot, c, b, w, true);
     return;
@@ -88,7 +88,7 @@ __device__ void run_world(int mslot, const myo_task_cfg& t, const BatchPtrs& b, 
     if (!io) return;
     phase_tree_forward<G>(mslot, c, false);
     task_obs<G>(mslot, t, c, ptarget);
-    for (int i = c.lane; i < m.nobs; i += G) a.obs[(size_t)w * m.nobs + i] = SF(o_obs)[i];
+    write_obs<G>(mslot, c, a.obs + (size_t)w * m.nobs, b.time + w, false);
     return;
   }
   if (a.mode == MODE_FORWARD || a.mode == MODE_MJ_STEP) {
@@ -121,6 +121,7 @@ __device__ void run_world(int mslot, const myo_task_cfg& t, const BatchPtrs& b, 
     float info[MYO_INFO_TERMS], reward;
     bool env_done;
     task_reward<G>(mslot, t, c, tf, ti[TI_ELAPSED] + 1, info, &reward, &env_done);
+    if (t.reward_sparse) reward = info[4];      // reward_mode "sparse": the sparse term, slot 4 of every kind
     // a world whose state left the finite range ends its episode here (MuJoCo would warn and reset the data): the reset
     // below keeps NaNs out of the running moments downstream
     bool bad = false;
@@ -132,7 +133,7 @@ __device__ void run_world(int mslot, const myo_task_cfg& t, const BatchPtrs& b, 
 #pragma unroll
       for (int k = 0; k < MYO_INFO_TERMS; k++) info[k] = 0.f;
       info[6] = 1.f;
-      for (int i = c.lane; i < m.nobs; i += G) SF(o_obs)[i] = 0.f;
+      for (int i = c.lane; i < m.nobs_scr; i += G) SF(o_obs)[i] = 0.f;
       c.tile.sync();
     }
     const int elapsed = ti[TI_ELAPSED] + 1;
@@ -150,7 +151,7 @@ __device__ void run_world(int mslot, const myo_task_cfg& t, const BatchPtrs& b, 
     }
     if (a.info && io) for (int k = c.lane; k < MYO_INFO_TERMS; k += G) a.info[(size_t)w * MYO_INFO_TERMS + k] = info[k];
     if (done && t.auto_reset) {
-      if (a.terminal_obs && io) for (int i = c.lane; i < m.nobs; i += G) a.terminal_obs[(size_t)w * m.nobs + i] = SF(o_obs)[i];
+      if (a.terminal_obs && io) write_obs<G>(mslot, c, a.terminal_obs + (size_t)w * m.nobs, b.time + w, bad);
       if (!SOLO && reset_needs_physics(t)) {
         // the reset runs an env step of its own (reference-state initialisation): done by a full-capacity pass, which also
         // writes the first observation of the new episode; the terminal state is stored as it is and the world is handed
@@ -163,7 +164,7 @@ __device__ void run_world(int mslot, const myo_task_cfg& t, const BatchPtrs& b, 
         task_obs<G>(mslot, t, c, ptarget);
       }
     }
-    if (io && !deferred_reset) for (int i = c.lane; i < m.nobs; i += G) a.obs[(size_t)w * m.nobs + i] = SF(o_obs)[i];
+    if (io && !deferred_reset) write_obs<G>(mslot, c, a.obs + (size_t)w * m.nobs, b.time + w, bad);
   }
   // status flags
   for (int i = c.lane; i < m.nq; i += G) if (!isfinite(SF(o_qpos)[i])) status |= ST_NONFINITE;

@@ -523,11 +523,59 @@ std::string pack_model(const Model& m, const myo_task_cfg& cfg, PackedModel& out
   B.F(d.d_invweight0, fvec(m, "dof_invweight0")); B.F(d.d_M0, fvec(m, "dof_M0"));
 
   // ---------------------------------------------------------------- task-dependent sizes
-  if (cfg.kind == MYO_TASK_BAODING) d.nobs = (nq - 14) + 24 + na;
-  else if (cfg.kind == MYO_TASK_POSE) d.nobs = nq + nv + nq + na;
-  else if (cfg.kind == MYO_TASK_REORIENT) d.nobs = (nq - 7) + (nv - 6) + 18 + na;
-  else if (cfg.kind == MYO_TASK_REACH) d.nobs = nq + nv + 6 * cfg.reach_nsite + na;      // qpos qvel*dt tip_pos reach_err act
-  else d.nobs = nq + nv + na;
+  // canonical observation (task_obs): the default obs_keys of the kind, each key's (first word, width) in it
+  std::vector<std::pair<int, int>> keys;      // indexed by MYO_OBS_<KIND>_* id; {-1, 1}: t
+  if (cfg.kind == MYO_TASK_BAODING) {
+    const int nh = nq - 14;
+    d.nobs_scr = nh + 24 + na;
+    keys = {{-1, 1}, {0, nh}};
+    for (int k = 0; k < 8; k++) keys.push_back({nh + 3 * k, 3});      // object1_pos .. target2_err
+    keys.push_back({nh + 24, na});
+  } else if (cfg.kind == MYO_TASK_POSE) {
+    d.nobs_scr = nq + nv + nq + na;
+    keys = {{-1, 1}, {0, nq}, {nq, nv}, {2 * nq + nv, na}, {nq + nv, nq}};      // t qpos qvel act pose_err
+  } else if (cfg.kind == MYO_TASK_REORIENT) {
+    const int nh = nq - 7, nhv = nv - 6, o0 = nh + nhv;
+    d.nobs_scr = o0 + 18 + na;
+    keys = {{-1, 1}, {0, nh}, {nh, nhv}};
+    for (int k = 0; k < 6; k++) keys.push_back({o0 + 3 * k, 3});       // obj_pos .. rot_err
+    keys.push_back({o0 + 18, na});
+  } else if (cfg.kind == MYO_TASK_REACH) {
+    const int o0 = nq + nv, w3 = 3 * cfg.reach_nsite;      // qpos qvel*dt tip_pos reach_err act
+    d.nobs_scr = o0 + 2 * w3 + na;
+    keys = {{-1, 1}, {0, nq}, {nq, nv}, {o0 + 2 * w3, na}, {o0, w3}, {-2, w3}, {o0 + w3, w3}};   // target_pos = tip_pos + reach_err
+  } else {
+    d.nobs_scr = nq + nv + na;
+  }
+  d.nobs = d.nobs_scr;
+  d.nobs_run = 0;
+  if (cfg.n_obs_keys != 0) {
+    if (cfg.n_obs_keys < 0 || cfg.n_obs_keys > MYO_MAX_OBS_KEYS) { status = MYO_E_LIMIT; return "obs_keys: 1 .. MYO_MAX_OBS_KEYS keys"; }
+    if (keys.empty()) { status = MYO_E_ARG; return "obs_keys: this task kind has no observation keys"; }
+    d.nobs = 0;
+    for (int k = 0; k < cfg.n_obs_keys; k++) {
+      const int id = cfg.obs_keys[k];
+      if (id < 0 || id >= (int)keys.size()) {
+        status = MYO_E_ARG;
+        return "obs_keys: key id " + std::to_string(id) + " is not one of this task kind's " + std::to_string(keys.size()) + " keys";
+      }
+      int src = keys[id].first, width = keys[id].second, op = OBS_RUN_COPY;
+      if (src == -1) { src = 0; op = OBS_RUN_TIME; }
+      else if (src == -2) { src = nq + nv; op = OBS_RUN_SUM; }
+      d.nobs += width;
+      if (width == 0) continue;
+      if (d.nobs_run > 0 && op == OBS_RUN_COPY) {
+        int& last = d.obs_run[d.nobs_run - 1];
+        const int lw = (last >> 16) & 0xfff;
+        if ((last >> 28) == OBS_RUN_COPY && (last & 0xffff) + lw == src && lw + width < 0x1000) {
+          last += width << 16;      // continues the previous run
+          continue;
+        }
+      }
+      if (src >= 0x10000 || width >= 0x1000) { status = MYO_E_LIMIT; return "obs_keys: observation too wide for the gather table"; }
+      d.obs_run[d.nobs_run++] = src | (width << 16) | (op << 28);
+    }
+  }
   d.nobs4 = pad4(d.nobs);
   {
     const double* q0 = m.d("qpos0");
@@ -620,7 +668,7 @@ std::string pack_model(const Model& m, const myo_task_cfg& cfg, PackedModel& out
         words = std::max(words, off - a0);
       }
       dd.o_obs = a0;
-      off = a0 + std::max(words, pad4(dd.nobs));
+      off = a0 + std::max(words, pad4(dd.nobs_scr));
     }
     dd.o_misc = take(MI_WORDS);
     // velocity-stage temporaries and the composite inertias are dead once M and qfrc_bias exist; the Newton Hessian

@@ -154,6 +154,29 @@ MYO_PHASE void task_obs(int mslot, const myo_task_cfg& t, Ctx<G, V> c, const flo
   c.tile.sync();
 }
 
+// the observation in the cfg's obs_keys layout, gathered from the canonical one in scratch (m.obs_run). time: the world's time,
+// written by lane 0 just before some of the calls; zero: a non-finite world, whose observation is all zeros, t included.
+template <int G, int V>
+MYO_PHASE void gather_obs(int mslot, Ctx<G, V> c, float* out, const float* time, bool zero) {
+  MYO_M
+  c.tile.sync();
+  const float tv = zero ? 0.f : *time;
+  const float* obs = SF(o_obs);
+  for (int r = 0, o = 0; r < m.nobs_run; r++) {
+    const int e = m.obs_run[r], src = e & 0xffff, n = (e >> 16) & 0xfff, op = e >> 28;
+    for (int i = c.lane; i < n; i += G)
+      out[o + i] = op == OBS_RUN_TIME ? tv : (op == OBS_RUN_SUM ? obs[src + i] + obs[src + n + i] : obs[src + i]);
+    o += n;
+  }
+}
+// obs out of scratch into out[nobs]: a straight copy for the default layout
+template <int G, int V>
+MYO_DI void write_obs(int mslot, Ctx<G, V> c, float* out, const float* time, bool zero) {
+  MYO_M
+  if (m.nobs_run == 0) for (int i = c.lane; i < m.nobs; i += G) out[i] = SF(o_obs)[i];
+  else gather_obs<G>(mslot, c, out, time, zero);
+}
+
 // ReachEnvV0.get_reward_dict from the observation in scratch: one distance over all 3 n entries of reach_err. ReachEnvV0 applies
 // far_th only once data.time > 2 dt; `elapsed` (env steps since the reset, this one included) stands in for the time.
 template <int G, int V>

@@ -50,6 +50,16 @@ class TaskClassifier:
             mean, scale = sc.mean_, sc.scale_
         return cls(sd, mean, scale, device)
 
+    @staticmethod
+    def check_env(env) -> None:
+        """The window is ``obs[29:47]`` of the default Baoding layout: refuse an env whose observation is laid out otherwise."""
+        from .vec_env import DEFAULT_OBS_KEYS
+
+        want = DEFAULT_OBS_KEYS[_capi.TASK_BAODING] + ("act",)
+        if env.cfg.kind != _capi.TASK_BAODING or getattr(env, "obs_keys", want) != want:
+            raise ValueError(f"the task classifier reads obs[{OBS_SLICE[0]}:{OBS_SLICE[1]}] of the default Baoding observation; this env's "
+                             f"observation is {list(env.obs_keys) if getattr(env, 'obs_keys', None) else 'not a Baoding one'}")
+
     def logits(self, window: torch.Tensor) -> torch.Tensor:
         """``window``: [n, 13 * 18] raw observations, step-major as ``np.concatenate(obs_for_classifier)`` lays them out."""
         x = (window.to(self.device, torch.float32) - self.mean) / self.scale
@@ -149,6 +159,8 @@ def evaluate_mixture(model, env, n_episodes: int = 2000, max_steps: Optional[int
     """``eval_perf``: episodes played back to back with the mixture's actions; mean length / reward with standard errors, mean
     effort (``|act| / na`` averaged per episode) and the classifier's error rate against the env's own task (``which_task`` of
     each world, clipped to hold / rotate). ``model``: ``MixtureOfEnsembles`` or ``Ensemble``; ``env``: ``MyoVecEnv`` (raw obs)."""
+    if isinstance(model, MixtureOfEnsembles):
+        TaskClassifier.check_env(env)
     n, dev = env.num_envs, env.device
     quota = max(1, math.ceil(n_episodes / n))
     obs = env.reset_device()

@@ -18,7 +18,7 @@ import numpy as np
 from . import _capi
 from .assets import asset_path
 from .sim import Model
-from .vec_env import BAODING_KEYS, POSE_KEYS, REACH_KEYS, REORIENT_KEYS, MyoVecEnv
+from .vec_env import BAODING_KEYS, OBS_KEYS, POSE_KEYS, REACH_KEYS, REORIENT_KEYS, MyoVecEnv
 
 _JNT_HAND = ['pro_sup', 'deviation', 'flexion', 'cmc_abduction', 'cmc_flexion', 'mp_flexion', 'ip_flexion', 'mcp2_flexion',
              'mcp2_abduction', 'pm2_flexion', 'md2_flexion', 'mcp3_flexion', 'mcp3_abduction', 'pm3_flexion', 'md3_flexion',
@@ -125,6 +125,27 @@ def _weights(cfg, keys, weighted_reward_keys):
         if k not in keys:
             raise ValueError(f"unknown reward key {k!r} (known: {keys})")
         cfg.rwd_weight[keys.index(k)] = float(w)
+
+
+def _obs_keys(cfg, model, obs_keys) -> None:
+    """MujocoEnv._setup's ``obs_keys``: the observation concatenates these obs-dict entries in order (duplicates allowed), and
+    BaseV0._setup appends "act" when the model has activations and the list lacks it."""
+    known = OBS_KEYS[cfg.kind]
+    if isinstance(obs_keys, str):
+        raise ValueError(f"obs_keys: a list of keys, got the string {obs_keys!r} (known: {list(known)})")
+    keys = list(obs_keys)
+    if not keys:
+        raise ValueError(f"obs_keys: empty list (known: {list(known)})")
+    unknown = [k for k in keys if k not in known]
+    if unknown:
+        raise ValueError(f"obs_keys: unknown key(s) {unknown} (known: {list(known)})")
+    if model.size("na") > 0 and "act" not in keys:
+        keys.append("act")
+    if len(keys) > _capi.MYO_MAX_OBS_KEYS:
+        raise ValueError(f"obs_keys: at most {_capi.MYO_MAX_OBS_KEYS} keys (\"act\" included), got {len(keys)}")
+    cfg.n_obs_keys = len(keys)
+    for i, k in enumerate(keys):
+        cfg.obs_keys[i] = known.index(k)
 
 
 def make_task_cfg(model: Model, env_id: str, **overrides) -> _capi.TaskCfg:
@@ -271,7 +292,13 @@ def make_task_cfg(model: Model, env_id: str, **overrides) -> _capi.TaskCfg:
             if gid >= 0:
                 cfg.n_ovr_geom, cfg.ovr_geom[0] = 1, gid
     kw.pop("model_path", None)
-    kw.pop("obs_keys", None)
+    obs_keys = kw.pop("obs_keys", None)
+    if obs_keys is not None:
+        _obs_keys(cfg, model, obs_keys)
+    reward_mode = kw.pop("reward_mode", "dense")
+    if reward_mode not in ("dense", "sparse"):
+        raise ValueError(f"reward_mode must be 'dense' or 'sparse', got {reward_mode!r}")
+    cfg.reward_sparse = int(reward_mode == "sparse")
     if kw:
         raise TypeError(f"unexpected env kwargs: {sorted(kw)}")
     return cfg

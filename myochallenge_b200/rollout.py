@@ -15,6 +15,7 @@ import numpy as np
 import torch
 
 from . import _capi
+from .vec_env import check_obs_width
 
 
 def _p(t):
@@ -214,6 +215,7 @@ class DeviceVecNormalize:
         from . import checkpoint
 
         st = checkpoint.load_vecnormalize(path)
+        check_obs_width(st["obs_mean"], venv.sim.nobs, path)
         vn = cls(venv, None, training=st["training"], norm_obs=st["norm_obs"], norm_reward=st["norm_reward"], clip_obs=st["clip_obs"],
                  clip_reward=st["clip_reward"], gamma=st["gamma"], epsilon=st["epsilon"])
         vn.obs_rms.load(st["obs_mean"], st["obs_var"], st["obs_count"])

@@ -78,6 +78,24 @@ REORIENT_KEYS = ("pos_dist", "rot_dist", "act_reg", "alive", "sparse", "solved",
 # MyoSuite ReachEnvV0.get_reward_dict [3P-MEM]
 REACH_KEYS = ("reach", "bonus", "act_reg", "penalty", "sparse", "solved", "done")
 
+# obs-dict entries of each task kind (get_obs_dict), numbered as the MYO_OBS_<KIND>_* ids of include/myo_b200.h: the keys `obs_keys`
+# may list
+OBS_KEYS = {
+    _capi.TASK_BAODING: ("t", "hand_pos", "object1_pos", "object1_velp", "object2_pos", "object2_velp", "target1_pos", "target2_pos",
+                         "target1_err", "target2_err", "act"),
+    _capi.TASK_REORIENT: ("t", "hand_qpos", "hand_qvel", "obj_pos", "goal_pos", "pos_err", "obj_rot", "goal_rot", "rot_err", "act"),
+    _capi.TASK_POSE: ("t", "qpos", "qvel", "act", "pose_err"),
+    _capi.TASK_REACH: ("t", "qpos", "qvel", "act", "tip_pos", "target_pos", "reach_err"),
+}
+# DEFAULT_OBS_KEYS of BaodingEnvV1, ReorientEnvV0, PoseEnvV0 and ReachEnvV0 (MyoSuite 1.2.3): the layout of an env created without
+# `obs_keys`, plus the "act" that BaseV0._setup appends for a model with activations
+DEFAULT_OBS_KEYS = {
+    _capi.TASK_BAODING: OBS_KEYS[_capi.TASK_BAODING][1:10],
+    _capi.TASK_REORIENT: OBS_KEYS[_capi.TASK_REORIENT][1:9],
+    _capi.TASK_POSE: ("qpos", "qvel", "pose_err"),
+    _capi.TASK_REACH: ("qpos", "qvel", "tip_pos", "reach_err"),
+}
+
 
 class MyoVecEnv:
     """SB3 ``VecEnv``-shaped front end over ``BatchSim``."""
@@ -95,6 +113,13 @@ class MyoVecEnv:
             raise ValueError(f"no reward keys for task kind {cfg.kind}")
         self._keys = keys[cfg.kind]
         self.info_keys = tuple(self._keys)      # names of the columns of ``sim.info`` (the reward terms ``infos[i]`` carries)
+        # the obs-dict entries the observation concatenates (None for a kind without keys)
+        if cfg.n_obs_keys:
+            self.obs_keys = tuple(OBS_KEYS[cfg.kind][cfg.obs_keys[i]] for i in range(cfg.n_obs_keys))
+        elif cfg.kind in DEFAULT_OBS_KEYS:
+            self.obs_keys = DEFAULT_OBS_KEYS[cfg.kind] + (("act",) if self.sim.na > 0 else ())
+        else:
+            self.obs_keys = None
         n, pin = self.num_envs, self.device.type == "cuda"
         self._h_act = torch.zeros(n, self.sim.nu, dtype=torch.float32, pin_memory=pin)
         self._h_obs = torch.zeros(n, self.sim.nobs, dtype=torch.float32, pin_memory=pin)
@@ -231,6 +256,13 @@ class RunningMeanStd:
         self.update_from_moments(mean.reshape(self.mean.shape), np.maximum(var, 0.0).reshape(self.var.shape), cnt)
 
 
+def check_obs_width(obs_mean, nobs: int, path: str) -> None:
+    """Observation statistics saved for one layout cannot normalise another (e.g. an env created with other ``obs_keys``)."""
+    d = int(np.asarray(obs_mean).size)
+    if d != int(nobs):
+        raise ValueError(f"{path}: the saved observation statistics are {d} wide, the env's observations {int(nobs)}")
+
+
 def rank_seed(base_seed: int, rank: int) -> int:
     """Seed of the worlds owned by ``rank``: world w of rank r draws from the stream (base + 1000 r, w, episode)."""
     return int(base_seed) + 1000 * int(rank)
@@ -269,6 +301,7 @@ class VecNormalize:
         from . import checkpoint
 
         st = checkpoint.load_vecnormalize(load_path)
+        check_obs_width(st["obs_mean"], venv.observation_space.shape[0], load_path)
         return cls.from_moments(venv, st["obs_mean"], st["obs_var"], st["obs_count"], st["ret_mean"], st["ret_var"], st["ret_count"],
                                 training=st["training"], norm_obs=st["norm_obs"], norm_reward=st["norm_reward"], clip_obs=st["clip_obs"],
                                 clip_reward=st["clip_reward"], gamma=st["gamma"], epsilon=st["epsilon"])
