@@ -233,7 +233,7 @@ __global__ void __launch_bounds__(kThreads) world_kernel(int mslot, int mslot_fu
   const int tid = threadIdx.x / G;
   c.soff = m.tab_words + tid * m.scratch_words;
   constexpr int RMAX = kFastRows / G > 0 ? kFastRows / G : 1;
-#if !defined(MYO_EMUL) && !defined(MYO_NO_HEAVY)
+#ifndef MYO_EMUL
   if (b.sched && a.mode == MODE_ENV_STEP) {
     // Env step with dynamic scheduling: groups of wpc worlds (in the sorted order: heavy worlds first) are fetched from a
     // global counter; when none is left the CTA serves the redo list - worlds that outgrew the fast layout, resets that run
@@ -242,7 +242,6 @@ __global__ void __launch_bounds__(kThreads) world_kernel(int mslot, int mslot_fu
     __shared__ int s_pick[3];
     const int ngroups = b.n_alloc / wpc;
     const DevModel& mf = c_models[mslot_full];
-    constexpr int RFULL = kSoloRowsPerLane;
     bool exhausted = false;      // (thread 0) no group of worlds is left in the queue
     for (;;) {
       if (threadIdx.x == 0) {
@@ -282,15 +281,7 @@ __global__ void __launch_bounds__(kThreads) world_kernel(int mslot, int mslot_fu
         int e;
         while ((e = ld_volatile(b.redo_list + idx + tid)) < 0) __nanosleep(200);      // reserved but not written yet
         __threadfence();
-#ifdef MYO_HEAVY_INLINE
-        Ctx<G, 1> ch(tile);
-        ch.soff = m.tab_words + tid * mf.scratch_words;
-        StepArgs ar = a;
-        ar.mode = MODE_REDO;
-        run_world<G, RFULL, true>(mslot_full, t, b, ar, ch, e & 0x3fffffff, e >> 30);
-#else
         heavy_world<G>(mslot_full, t, b, a, m.tab_words + tid * mf.scratch_words, e);
-#endif
       }
     }
     return;
@@ -452,6 +443,14 @@ __global__ void repack_kernel(float* dst, int dst_stride, int dst_off, const flo
 }  // namespace myo
 
 // ------------------------------------------------------------------------------------------------
+// The redo of worlds the fast layout cannot finish runs inside the fast kernel (dynamic scheduling) on the device; the host
+// emulation has no such scheduler and runs it as a separate pass of the solo kernel.
+#ifdef MYO_EMUL
+constexpr bool kDynSched = false;
+#else
+constexpr bool kDynSched = true;
+#endif
+
 struct myo_batch {
   myo::PackedModel pm;
   myo_task_cfg cfg;
@@ -460,8 +459,6 @@ struct myo_batch {
   int grid = 0, threads = myo::kThreads, smem = 0, regs = 0, wpc = 0, tab_bytes = 0;
   int solo_grid = 0, solo_smem = 0, solo_regs = 0;
   bool use_redo = false;       // worlds the fast layout cannot finish are redone with full capacities within the same env step
-  bool dyn_sched = false;      // ... inside the fast kernel (dynamic scheduling); false: by a separate pass of the solo kernel
-  int* sched_dev = nullptr;
   int64_t launches = 0;
   std::vector<void*> allocs;
   // world grouping: after every env step the worlds are sorted by the constraint rows of their last substep, and the next
@@ -567,7 +564,6 @@ template <int G> int configure(myo_batch* b) {
   const size_t max_smem = prop.sharedMemPerBlockOptin - tab_bytes;
   // worlds per CTA: fill the SM's shared memory with as few CTAs as keep threads <= kThreads
   int wpc = kThreads / G;
-  if (const char* ov = getenv("MYO_WPC")) { const int v = atoi(ov); if (v >= 1 && v < wpc) wpc = v; }   // development override
   while (wpc > 1 && wpc * world_bytes > max_smem) wpc--;
   if (wpc * world_bytes > max_smem) { set_error("one world's scratch exceeds shared memory per CTA"); return MYO_E_LIMIT; }
   // a batch smaller than one CTA steps no padding worlds beside its own; the CTA keeps room for one full-capacity world (redo)
@@ -773,27 +769,17 @@ int myo_batch_create(const myo_model* mh, int n_worlds, int device, const myo_ta
   b->p.redo_list = nullptr; b->p.redo_count = nullptr;
   {
     // the full-capacity pass after every env step is needed when the fast layout is smaller than MuJoCo's capacities or
-    // when resets run physics (MYO_REDO=0 switches it off for experiments: overflowing worlds are then truncated + flagged)
+    // when resets run physics
     const myo::DevModel& df = b->pm.dm_full;
-    bool want = df.ncon_max > dm.ncon_max || df.nlim_max > dm.nlim_max || df.nefc_max > dm.nefc_max || myo::reset_needs_physics(*cfg);
-    if (const char* e = getenv("MYO_REDO")) want = want && atoi(e) != 0;
-    b->use_redo = want;
+    b->use_redo = df.ncon_max > dm.ncon_max || df.nlim_max > dm.nlim_max || df.nefc_max > dm.nefc_max || myo::reset_needs_physics(*cfg);
     if ((rc = dev_alloc(b, &b->p.redo_list, n)) || (rc = dev_alloc(b, &b->p.redo_count, 4)) || (rc = dev_alloc(b, &b->p.sched, 4))) return fail(rc);
-    if (!want) b->p.redo_list = nullptr;
+    if (!b->use_redo) b->p.redo_list = nullptr;
     b->p.heavy_per_cta = std::max(1, std::min(b->wpc, (int)((b->smem - b->tab_bytes) / ((size_t)df.scratch_words * sizeof(float)))));
-#if defined(MYO_EMUL) || defined(MYO_NO_HEAVY)
-    b->dyn_sched = false;
-#else
-    b->dyn_sched = true;
-    if (const char* e = getenv("MYO_DYN_SCHED")) b->dyn_sched = atoi(e) != 0;      // 0: static striding + a separate full-capacity pass
-#endif
-    b->sched_dev = b->p.sched;
-    if (!b->dyn_sched) b->p.sched = nullptr;
+    if (!kDynSched) b->p.sched = nullptr;
   }
 #ifndef MYO_EMUL
   {
-    const char* e = getenv("MYO_SORT_WORLDS");
-    b->sort_worlds = e ? atoi(e) != 0 : (b->p.n_alloc >= 4 * b->wpc * 148);      // worth it only when every SM sees several groups
+    b->sort_worlds = b->p.n_alloc >= 4 * b->wpc * 148;      // worth it only when every SM sees several groups
     if (b->sort_worlds) {
       if ((rc = dev_alloc(b, &b->p.work, n)) || (rc = dev_alloc(b, &b->order[0], n)) || (rc = dev_alloc(b, &b->order[1], n)) ||
           (rc = dev_alloc(b, &b->iota, n)) || (rc = dev_alloc(b, &b->keys_out, n)))
@@ -864,12 +850,12 @@ int myo_batch_step(myo_batch* b, const float* actions_dev, float* obs_dev, float
   cudaStream_t st_ = static_cast<cudaStream_t>(stream);
   if (b->use_redo) {
     CK(cudaMemsetAsync(b->p.redo_count, 0, sizeof(int), st_));
-    if (b->dyn_sched) CK(cudaMemsetAsync(b->p.redo_list, 0xFF, (size_t)b->p.n_alloc * sizeof(int), st_));
+    if (kDynSched) CK(cudaMemsetAsync(b->p.redo_list, 0xFF, (size_t)b->p.n_alloc * sizeof(int), st_));
   }
-  if (b->dyn_sched) CK(cudaMemsetAsync(b->sched_dev, 0, 4 * sizeof(int), st_));
+  if (kDynSched) CK(cudaMemsetAsync(b->p.sched, 0, 4 * sizeof(int), st_));
   int rc = launch(b, a, stream);
   b->p.order = nullptr;
-  if (!rc && b->use_redo && !b->dyn_sched) {      // worlds the fast kernel could not finish: same step, full capacities, one world per CTA
+  if (!rc && b->use_redo && !kDynSched) {      // worlds the fast kernel could not finish: same step, full capacities, one world per CTA
     a.mode = myo::MODE_REDO;
     rc = launch_full(b, a, stream);
   }

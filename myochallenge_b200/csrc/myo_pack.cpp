@@ -604,7 +604,7 @@ std::string pack_model(const Model& m, const myo_task_cfg& cfg, PackedModel& out
   { std::vector<int> tl = ivec(m, "tendon_limited"); for (int t = 0; t < ntendon; t++) if (tl[t]) { nlim++; d.any_tendon_limit = 1; } }
   if (nv > 64) { status = MYO_E_LIMIT; return "nv exceeds the dense solver limit (64)"; }
   out.lanes = nv <= 8 ? 8 : (nv <= 16 ? 16 : 32);
-  if (const char* ov = getenv("MYO_LANES")) {   // development override of the tile width (8, 16 or 32)
+  if (const char* ov = getenv("MYO_LANES")) {   // test hook: override of the tile width (8, 16 or 32), so that tests cover every instantiation
     const int g = atoi(ov);
     if (g == 8 || g == 16 || g == 32) out.lanes = g;
   }
@@ -624,9 +624,7 @@ std::string pack_model(const Model& m, const myo_task_cfg& cfg, PackedModel& out
     for (int a = 0; a < KS; a++) for (int b2 = 0; b2 <= a; b2++) pair_ab.push_back(a | (b2 << 8));
     B.I(d.pair_ab, pair_ab);
   }
-  int ncon_fast = 16, nlim_fast = 32;
-  if (const char* ov = getenv("MYO_NCON_CAP")) { const int v = atoi(ov); if (v >= 1 && v <= 16) ncon_fast = v; }     // development: fast-layout capacities
-  if (const char* ov = getenv("MYO_NLIM_CAP")) { const int v = atoi(ov); if (v >= 1 && v <= 32) nlim_fast = v; }
+  const int ncon_fast = 16, nlim_fast = 32;      // fast-layout capacities
   B.finish();
   const int njmax = std::max(1, m.sz("njmax")), nconmax = std::max(1, m.sz("nconmax"));
   // alias: the fast layout, which only the env step (and reset / get_obs, which run no physics) uses. Words of vectors

@@ -350,12 +350,7 @@ MYO_PHASE void mul_M(int mslot, Ctx<G, V> c, int oM, int ox, int oy, bool sync =
 
 // Helpers that take pointers to the caller's small arrays (points, frames, coefficient sets): as noinline functions those arrays
 // live in local memory and every call stores and reloads them (round-2 profile: 240 local loads + 90 local stores per world
-// and substep, 1.85 of 32 bytes used per sector). Inlined, they stay in registers. -DMYO_OUTLINE_HELPERS restores the calls.
-#ifdef MYO_OUTLINE_HELPERS
-#define MYO_HELPER MYO_PHASE
-#else
-#define MYO_HELPER MYO_DI
-#endif
+// and substep, 1.85 of 32 bytes used per sector). Inlined, they stay in registers.
 
 // ------------------------------------------------------------------------------------------------
 // a10.2 tendon length + moment arms (mj_tendon + mju_wrap), one lane per tendon.
@@ -377,7 +372,7 @@ MYO_DI bool seg_intersect(const float* p1, const float* p2, const float* p3, con
 }
 // 2-D wrap around a circle (MuJoCo wrap_circle). Arc angle via atan2(|cross|, dot): same value as
 // MuJoCo's acos(dot) but well conditioned in fp32 for small arcs.
-MYO_HELPER float wrap_circle(float* pnt, const float* d, const float* sd, float rad) {
+MYO_DI float wrap_circle(float* pnt, const float* d, const float* sd, float rad) {
   const float sqlen0 = d[0] * d[0] + d[1] * d[1], sqlen1 = d[2] * d[2] + d[3] * d[3], sqrad = rad * rad;
   const float dif[2] = {d[2] - d[0], d[3] - d[1]};
   const float dd = dif[0] * dif[0] + dif[1] * dif[1];
@@ -419,8 +414,8 @@ MYO_HELPER float wrap_circle(float* pnt, const float* d, const float* sd, float 
   return rad * angle;
 }
 // returns curved length (>= 0) and two world points in wpnt[0..5]; -1 no wrap; -2 unsupported (inside wrap)
-MYO_HELPER float wrap_geom(float* wpnt, const float* x0, const float* x1, const float* gpos, const float* gmat, float radius,
-                           int type, const float* side) {
+MYO_DI float wrap_geom(float* wpnt, const float* x0, const float* x1, const float* gpos, const float* gmat, float radius,
+                       int type, const float* side) {
   float p0[3], p1[3], dif[3], axis0[3], axis1[3], normal[3];
   sub3(dif, x0, gpos); mulmatTvec3(p0, gmat, dif);
   sub3(dif, x1, gpos); mulmatTvec3(p1, gmat, dif);
@@ -488,7 +483,7 @@ MYO_DI int common_prefix(const DevModel& m, int ba, int bb) {
 // for the dofs on either body's chain past their common prefix (- on the pa side, + on the pb side). The dof list of the
 // (body, body) pair is precomputed (myo_pack.cpp seg_list): header n | rootA << 8 | rootB << 20, entries
 // dof | slot << 8 | end << 16, slot = position in the tendon's dof list = position in the segment's result row.
-MYO_HELPER void segment_moment(int mslot, int soff, int list, const float* pa, const float* pb, float inv_div, float* out) {
+MYO_DI void segment_moment(int mslot, int soff, int list, const float* pa, const float* pb, float inv_div, float* out) {
   MYO_M
   if (list < 0) return;
   const float* s = MYO_SMEM_WORDS + soff;
@@ -919,8 +914,8 @@ MYO_PHASE void phase_collision(int mslot, Ctx<G, V> c, int* status) {
 }
 
 // impedance, regularisation and reference-acceleration coefficients of one row (mj_makeImpedance)
-MYO_HELPER void row_params(int mslot, const float* solref, const float* solimp, float pos, float margin, float diag,
-                       float* R, float* K, float* B, float* imp) {
+MYO_DI void row_params(int mslot, const float* solref, const float* solimp, float pos, float margin, float diag,
+                   float* R, float* K, float* B, float* imp) {
   MYO_M
   const float s0 = clipf(solimp[0], 0.0001f, 0.9999f), s1 = clipf(solimp[1], 0.0001f, 0.9999f);
   const float s2 = fmaxf(0.f, solimp[2]), s3 = clipf(solimp[3], 0.0001f, 0.9999f), s4 = fmaxf(1.f, solimp[4]);
@@ -1727,44 +1722,11 @@ MYO_PHASE void solve_M_dense(int mslot, Ctx<G, V> c, int ox, float hdamp) {
 // All warps of a CTA walk the phases together: the step is ~200 KB of straight-line code, far more
 // than the instruction cache holds, so keeping the CTA inside one phase at a time lets every fetched
 // line serve all of its warps. (Every tile of the CTA executes every phase of every substep.)
-#ifndef MYO_LOCKSTEP_WARPS
-#define MYO_LOCKSTEP_WARPS 0      // 0: the whole CTA walks the phases together; k: groups of k warps do (named barriers)
-#endif
-MYO_DI void lockstep_sync() {
-#if defined(MYO_EMUL) || MYO_LOCKSTEP_WARPS == 0
-  __syncthreads();
-#else
-  const unsigned nw = blockDim.x >> 5;
-  if (nw % MYO_LOCKSTEP_WARPS) { __syncthreads(); return; }
-  const unsigned group = (threadIdx.x >> 5) / MYO_LOCKSTEP_WARPS;
-  asm volatile("bar.sync %0, %1;" ::"r"(1u + group), "r"(32u * MYO_LOCKSTEP_WARPS) : "memory");
-#endif
-}
-#define MYO_CTA_SYNC lockstep_sync();
-// which of the eight phase boundaries of a substep carry the CTA barrier (bit i = boundary before phase i in the order
-// tree_forward, mass_bias, tendon, collision, constraints, actuation, solve, integrate). Worlds are independent, so the
-// barriers are a performance device only (instruction-cache sharing); see DESIGN.md for the measured choices.
-#ifndef MYO_SYNC_MASK
-#define MYO_SYNC_MASK 0xFF
-#endif
-#define MYO_SYNC(i) if (SYNC && ((MYO_SYNC_MASK >> (i)) & 1)) lockstep_sync();      // SYNC: template flag of the step functions
+// Every phase boundary of a substep carries the CTA barrier. Worlds are independent, so the barriers are a performance
+// device only (instruction-cache sharing); see DESIGN.md for the measured choices.
+#define MYO_SYNC if (SYNC) __syncthreads();      // SYNC: template flag of the step functions
 
-// Optional (MYO_NEWTON_LOCKSTEP=1): the Newton iterations of a CTA's worlds in lock step too - barriers between Hessian build,
-// factorisation and line search, a CTA-wide vote ending the loop when no world iterates. Measured 3 % SLOWER than letting
-// each world iterate freely inside the phase (28.5 vs 27.7 ms per 32768-world step at steady state), so it is off.
-#ifndef MYO_NEWTON_LOCKSTEP
-#define MYO_NEWTON_LOCKSTEP 0
-#endif
-#ifndef MYO_NEWTON_STEP_TOL
-#define MYO_NEWTON_STEP_TOL 2e-5f      // last Newton step relative to max(1, |qacc|_inf) below which the solve stops (fp32 floor)
-#endif
-MYO_DI bool cta_any(bool v) {
-#if defined(MYO_EMUL)
-  return v;
-#else
-  return __syncthreads_or(v ? 1 : 0) != 0;
-#endif
-}
+constexpr float kNewtonStepTol = 2e-5f;      // last Newton step relative to max(1, |qacc|_inf) below which the solve stops (fp32 floor)
 template <int G, int RMAX, int V>
 MYO_PHASE void phase_solve(int mslot, Ctx<G, V> c, bool fast) {
   MYO_M
@@ -1778,7 +1740,7 @@ MYO_PHASE void phase_solve(int mslot, Ctx<G, V> c, bool fast) {
     for (int i = c.lane; i < nv; i += G) { a[i] = as[i]; SF(o_warm)[i] = as[i]; qcon[i] = 0.f; }
     if (c.lane == 0) misc[MI_ITER] = 0;
     c.tile.sync();
-    if (!MYO_NEWTON_LOCKSTEP) return;
+    return;
   }
   float* Ma = SF(o_Ma); float* grad = SF(o_grad); float* p = SF(o_p); float* Mp = SF(o_Mp);
   // constraint rows in registers for the reductions and the line search: lane owns rows lane, lane + G, ...
@@ -1827,27 +1789,18 @@ MYO_PHASE void phase_solve(int mslot, Ctx<G, V> c, bool fast) {
   }
   const float scale = 1.f / (m.meaninertia * (float)max(1, nv));
   int iter = 0;
-  int exit_reason = 0;
-#ifdef MYO_EXIT_STATS
-#define MYO_EXIT_REASON(r) exit_reason = (r);
-#else
-#define MYO_EXIT_REASON(r)
-#endif
   MYO_PH_BEGIN
   float prev_step = 3.0e38f;
   for (int it = 0; it < m.solver_iter; it++) {
-    if (MYO_NEWTON_LOCKSTEP) { if (!cta_any(active)) break; }
-    else if (!active) break;
+    if (!active) break;
     if (active) {
       MYO_PH_RESTART newton_system<G>(mslot, c); MYO_PH(11)
       float g2 = 0.f;
       for (int i = c.lane; i < nv; i += G) g2 += grad[i] * grad[i];
       g2 = tile_sum<G>(c, g2);
-      if (sqrtf(g2) * scale < m.solver_tol) { active = false; MYO_EXIT_REASON(4) }
+      if (sqrtf(g2) * scale < m.solver_tol) active = false;
     }
-    if (MYO_NEWTON_LOCKSTEP) lockstep_sync();
     if (active) { chol_factor_solve<G>(mslot, c, m.o_H, m.o_p, nv); MYO_PH(12) }
-    if (MYO_NEWTON_LOCKSTEP) lockstep_sync();
     if (active) {
     rows_dot<G>(mslot, c, m.o_p, R_JP, false, false);
     mul_M<G>(mslot, c, m.o_M, m.o_p, m.o_Mp);
@@ -1896,14 +1849,13 @@ MYO_PHASE void phase_solve(int mslot, Ctx<G, V> c, bool fast) {
     for (int i = c.lane; i < nv; i += G) { a[i] += alpha * p[i]; Ma[i] += alpha * Mp[i]; }
     c.tile.sync();
     iter++;
-    if (!changed && fabsf(alpha - 1.f) <= 1e-3f) { active = false; MYO_EXIT_REASON(1) }
-#ifdef MYO_SOLVER_DEBUG
-    if (iter > 9) printf("it %d alpha %.6f pmax %.3e amax %.3e gp %.3e pMp %.3e nefc %d\n", iter, alpha, pmax, amax, gp, pMp, nefc);
-#endif
+    if (!changed && fabsf(alpha - 1.f) <= 1e-3f) active = false;
     // fp32 termination: the Newton step is at the rounding floor of qacc (quadratic convergence makes
-    // the remaining error far smaller than the last step), or it stopped shrinking (noise-level cycling)
+    // the remaining error far smaller than the last step), or it stopped shrinking (noise-level cycling).
+    // The empty `if (active)` is kept on purpose: without it the compiler lays the solve out differently, and the kernels
+    // built from this phase get larger stack frames and more spills (world_kernel<32>: 512 -> 528 B of stack).
     const float step = alpha * pmax, aref_mag = fmaxf(1.f, amax);
-    if (step <= MYO_NEWTON_STEP_TOL * aref_mag || (iter > 1 && step >= 0.5f * prev_step && step <= 1e-3f * aref_mag)) { if (active) { MYO_EXIT_REASON(step <= MYO_NEWTON_STEP_TOL * aref_mag ? 2 : 3) } active = false; }
+    if (step <= kNewtonStepTol * aref_mag || (iter > 1 && step >= 0.5f * prev_step && step <= 1e-3f * aref_mag)) { if (active) {} active = false; }
     prev_step = step;
     }
   }
@@ -1912,7 +1864,7 @@ MYO_PHASE void phase_solve(int mslot, Ctx<G, V> c, bool fast) {
   for (int i = c.lane; i < nv; i += G) { qcon[i] = 0.f; SF(o_warm)[i] = a[i]; }
   c.tile.sync();
   rows_JT_force<G>(mslot, c, m.o_qcon, 1.f);
-  if (c.lane == 0) misc[MI_ITER] = iter + (exit_reason << 8);
+  if (c.lane == 0) misc[MI_ITER] = iter;
   c.tile.sync();
 }
 
@@ -1964,24 +1916,24 @@ template <int G, int RMAX, bool SYNC, int V>
 MYO_PHASE void mj_forward_dev(int mslot, Ctx<G, V> c, int* status, bool fast) {
   MYO_M
   MYO_PH_BEGIN
-  MYO_SYNC(0) phase_tree_forward<G>(mslot, c, true); MYO_PH(0)
+  MYO_SYNC phase_tree_forward<G>(mslot, c, true); MYO_PH(0)
   MYO_PH(2)
-  MYO_SYNC(1) phase_mass_bias<G>(mslot, c); MYO_PH(3)
+  MYO_SYNC phase_mass_bias<G>(mslot, c); MYO_PH(3)
   // the velocity-stage temporaries are dead from here on: the tendon phase reuses their scratch (with the Hessian's)
-  MYO_SYNC(2) phase_tendon<G>(mslot, c, status); MYO_PH(1)
-  MYO_SYNC(3) phase_collision<G>(mslot, c, status); MYO_PH(5)
-  MYO_SYNC(4) phase_constraints<G>(mslot, c, status); MYO_PH(6)
-  MYO_SYNC(5) phase_actuation<G>(mslot, c); MYO_PH(7)
+  MYO_SYNC phase_tendon<G>(mslot, c, status); MYO_PH(1)
+  MYO_SYNC phase_collision<G>(mslot, c, status); MYO_PH(5)
+  MYO_SYNC phase_constraints<G>(mslot, c, status); MYO_PH(6)
+  MYO_SYNC phase_actuation<G>(mslot, c); MYO_PH(7)
   if (!fast || SI(o_misc)[MI_NEFC] == 0) solve_M_dense<G>(mslot, c, m.o_qaccs, 0.f);   // qacc_smooth (see phase_solve)
   MYO_PH(8)
-  MYO_SYNC(6) phase_solve<G, RMAX>(mslot, c, fast); MYO_PH(9)
+  MYO_SYNC phase_solve<G, RMAX>(mslot, c, fast); MYO_PH(9)
 }
 template <int G, int RMAX, bool SYNC, int V>
 MYO_PHASE void mj_step_dev(int mslot, Ctx<G, V> c, int* status, bool fast) {
   MYO_M
   mj_forward_dev<G, RMAX, SYNC>(mslot, c, status, fast);
   MYO_PH_BEGIN
-  MYO_SYNC(7) MYO_PH(15) phase_integrate<G>(mslot, c); MYO_PH(10)
+  MYO_SYNC MYO_PH(15) phase_integrate<G>(mslot, c); MYO_PH(10)
 }
 
 }  // namespace myo

@@ -63,7 +63,7 @@ struct NetProgram {
 };
 
 struct FwdArgs {
-  int n, obs_dim, obs_pad, H, act_dim, swap_lbo_sbo;
+  int n, obs_dim, obs_pad, H, act_dim;
   const float* obs;
   float* h;
   float* c;
@@ -405,8 +405,8 @@ policy_forward_kernel(const __grid_constant__ FwdArgs a, const __grid_constant__
           for (int ks = 0; ks < ck; ks += 16) {
             const uint32_t a_addr = a_base + (uint32_t)((k0 + ks) >> 3) * a_lbo;
             const uint32_t b_addr = b_base + (uint32_t)(ks >> 3) * b_lbo;
-            const uint64_t ad = a.swap_lbo_sbo ? make_desc(a_addr, 128, a_lbo) : make_desc(a_addr, a_lbo, 128);
-            const uint64_t bd = a.swap_lbo_sbo ? make_desc(b_addr, 128, b_lbo) : make_desc(b_addr, b_lbo, 128);
+            const uint64_t ad = make_desc(a_addr, a_lbo, 128);
+            const uint64_t bd = make_desc(b_addr, b_lbo, 128);
             umma_bf16(d_tmem, ad, bd, idesc, (k0 + ks) > 0 ? 1u : 0u);
           }
           umma_commit(bar_empty + 8 * s);
@@ -526,7 +526,6 @@ struct myo_policy {
   float clip_obs = 10.f;
   bool has_norm = false, dirty = true;
   unsigned long long seed = 0, step = 0;
-  int swap_lbo_sbo = 0;
   int64_t launches = 0;
   float* latent_out = nullptr;   // caller-owned [max_batch][latent_dim], see myo_policy_set_latent_out
   // fp32 mode (myo_policy_set_precision): plain SGEMMs on the fp32 weights + elementwise kernels, for evaluating trained
@@ -787,7 +786,6 @@ int myo_policy_create(const myo_policy_cfg* cfg, int max_batch, int device, myo_
   PCK(cudaSetDevice(device));
   myo_policy* p = new myo_policy();
   p->cfg = *cfg; p->device = device; p->max_batch = max_batch; p->obs_pad = round_up(cfg->obs_dim, 16);
-  if (const char* e = getenv("MYO_POLICY_SWAP_LBO_SBO")) p->swap_lbo_sbo = atoi(e);
   for (int net = 0; net < 2; net++) {
     build_program(p, net, p->prog[net], p->wbytes[net], p->nbias[net]);
     if (cudaMalloc(&p->wpack[net], p->wbytes[net]) != cudaSuccess || cudaMalloc(&p->bias[net], sizeof(float) * p->nbias[net]) != cudaSuccess) {
@@ -877,7 +875,6 @@ int myo_policy_forward(myo_policy* p, int n, const float* obs_dev, float* h_dev,
   if (p->dirty) { int rc = pack_weights(p, st); if (rc) return rc; }
   FwdArgs a{};
   a.n = n; a.obs_dim = p->cfg.obs_dim; a.obs_pad = p->obs_pad; a.H = p->cfg.lstm_hidden; a.act_dim = p->cfg.act_dim;
-  a.swap_lbo_sbo = p->swap_lbo_sbo;
   a.obs = obs_dev; a.h = h_dev; a.c = c_dev; a.start = episode_start_dev; a.noise = noise_dev;
   a.actions = actions_dev; a.values = values_dev; a.logp = logp_dev;
   a.wpack[0] = p->wpack[0]; a.wpack[1] = p->wpack[1]; a.bias[0] = p->bias[0]; a.bias[1] = p->bias[1];

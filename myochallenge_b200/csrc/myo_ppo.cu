@@ -590,7 +590,7 @@ struct myo_ppo {
   // captured once into a CUDA graph (about 1 100 short launches) and replayed while the arguments stay the same
   cudaStream_t side = nullptr, main = nullptr;     // main: the graph's origin stream (the caller's may be the legacy default stream, which cannot be captured)
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr, ev_in = nullptr, ev_out = nullptr;
-  bool use_graph = true, have_graph = false;
+  bool have_graph = false;
   long long* seq_prof = nullptr;     // MYO_PPO_SEQ_PROF=1: cycle counters of the forward cluster kernel (development)
   bool use_seq = false;              // bf16 mode with a supported hidden size: the recurrence runs in the persistent cluster kernels
   cudaGraphExec_t exec = nullptr;
@@ -868,7 +868,6 @@ GradKey make_key(const GradArgs& a) {
 template <typename T>
 int minibatch_grad(myo_ppo* p, const GradArgs& a, cudaStream_t st) {
   QCK(cudaMemcpyAsync(p->idx, a.idx, sizeof(int32_t) * a.B, cudaMemcpyDeviceToDevice, st));
-  if (!p->use_graph) return minibatch_issue<T>(p, a, st);
   // the graph runs on the handle's own stream, ordered after / before the caller's stream by events
   QCK(cudaEventRecord(p->ev_in, st));
   QCK(cudaStreamWaitEvent(p->main, p->ev_in, 0));
@@ -972,7 +971,6 @@ int myo_ppo_create(const myo_policy_cfg* cfg, int max_steps, int max_worlds, int
     myo_ppo_destroy(p);
     return MYO_E_CUDA;
   }
-  if (const char* e = getenv("MYO_PPO_NO_GRAPH")) p->use_graph = atoi(e) == 0;
   *out = p;
   return MYO_OK;
 }
